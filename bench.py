@@ -4,6 +4,7 @@
   python bench.py --gpus N --steps K --warmup W                  # headline: BASELINE configs[1]
   python bench.py --workload pendulum|scale1m|equiv|cnn ...      # configs[2], configs[4], configs[3], its plain-CNN sibling
   python bench.py --impl reference [--workload ...] ...          # the reference's CPU path (oracle port), bounded sample
+  python bench.py ... --dump-outputs DIR                         # also write the last timed step's outputs as DIR/<name>.npy
 
 Workloads (SURVEY.md section 8, sizes per BASELINE.json):
   ppo       CartPole-v1, 65536 envs PER GPU (weak scaling), T = 128, 4 minibatches x 4 epochs           configs[1]
@@ -48,6 +49,31 @@ GAE_SWEEP_COLS = 131072                              # config E at 8 GPUs: 1M / 
 
 def num_envs_for(w, n_gpus):
     return w["total_envs"] if w["total_envs"] else w["envs_per_gpu"] * n_gpus
+
+
+# --dump-outputs: a larger output is written as a fixed sample, so that the whole dump stays small (well under 64 MB)
+DUMP_COLUMNS = 2048            # env columns of the [T, N, ...] rollout / GAE arrays
+DUMP_ELEMENTS = 1 << 20        # elements of any other array
+
+
+def seeded_sample(n, k):
+    """k of range(n), sorted; the same for every run and build (seed 0)."""
+    import torch
+    if n <= k:
+        return torch.arange(n)
+    return torch.randperm(n, generator=torch.Generator().manual_seed(0))[:k].sort().values
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor as out_dir/<name>.npy: float64 stays float64, every other dtype becomes float32."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_ELEMENTS:
+            t = t.reshape(-1)[seeded_sample(t.numel(), DUMP_ELEMENTS).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.to(torch.float64 if t.dtype == torch.float64 else torch.float32).cpu().numpy())
 
 
 HIDDEN = 64        # --hidden_dim (src/run_ppo.py:36): 64 is the reference default and every BASELINE config; 128 / 256 run the wide kernels
@@ -332,6 +358,7 @@ def run_ours(args):
         dist.init_process_group("nccl", device_id=torch.device(f"cuda:{local_rank}"))
     from aur_ppo_b200.ppo import ppo
     n_gpus = world
+    torch.manual_seed(1)            # the initial policy comes from torch's generator: every run starts from the same weights
     agent = ppo(params(name, n_gpus, args.steps + args.warmup))
     n_mb_iter = EPOCHS * math.ceil(agent.local_batch / agent.local_minibatch)
     agent._stats_rows = torch.zeros(n_mb_iter, 16, device=agent.device)
@@ -379,6 +406,13 @@ def run_ours(args):
                               "waits ~0, the others wait for it), and the spin time of the gradient kernels' CTAs on the moment flags "
                               "(only the first minibatch of an iteration can spin: the moments travel once per iteration)"}
     clocks = sampler.finish()
+    if args.dump_outputs and rank == 0:             # the last timed iteration, before the e2e loop below moves the agent on
+        b, cols = agent.buffer, seeded_sample(agent.local_envs, DUMP_COLUMNS).to(agent.device)
+        dump_outputs(args.dump_outputs, {
+            "params": agent.flat, "stats": agent._stats_rows, "obs": b.states[:, cols], "actions": b.actions[:, cols],
+            "log_probs": b.log_probs[:, cols], "values": b.values[:, cols], "rewards": b.rewards[:, cols],
+            "dones": b.terminals[:, cols], "next_value": b.next_value[cols], "returns": agent._returns[:, cols],
+            "advantages": agent._advantages[:, cols]})
     ms_total = start.elapsed_time(end)
     t_roll = sum(e[0].elapsed_time(e[1]) for e in ev) / args.steps
     t_gae = sum(e[1].elapsed_time(e[2]) for e in ev) / args.steps
@@ -605,11 +639,13 @@ def run_equiv(args, plain: bool = False):
     t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t0.record()
     for _ in range(args.steps):
-        model.update(state, obs, action, oldlp, adv, ret, vold)
+        st = model.update(state, obs, action, oldlp, adv, ret, vold)
     t1.record()
     torch.cuda.synchronize()
     launches = int(L.aur_launch_count())
     clocks = sampler.finish()
+    if args.dump_outputs:                           # the last timed update, before the e2e loop below runs more of them
+        dump_outputs(args.dump_outputs, {"params": model._flat["p"], "stats": st, "values": model.value, "log_probs": model.logp})
     ms = t0.elapsed_time(t1) / args.steps
     # e2e: observations, states, actions and targets uploaded from pinned host memory every step, stats read back
     # Two device buffer sets and a copy stream: the upload of step i+1 (269 MB of observations) runs while step i computes;
@@ -738,7 +774,14 @@ def main():
                          "planes (~5e-6 per layer); bf16 = single-plane fast mode, below the reference's precision")
     ap.add_argument("--hidden_dim", type=int, default=64, choices=[64, 128, 256],
                     help="policy width of the MLP workloads (src/run_ppo.py:36); 64 is every BASELINE config, 128 / 256 exercise the wide kernels")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32 / float64; "
+                         "large arrays as a fixed sample) so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     global HIDDEN
     HIDDEN = args.hidden_dim
     if args.warmup < 3 and args.impl == "ours":

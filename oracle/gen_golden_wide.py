@@ -5,7 +5,9 @@ not exist on the GPU box):  python oracle/gen_golden_wide.py  ->  tests/golden/u
 
 TEST INFRASTRUCTURE ONLY.  To keep the fixture small the initial parameters are NOT stored: they are gen_golden.fill_params'
 closed form (i-th parameter tensor <- 0.1 sin(0.37 k + i)), which the test re-creates from the stored parameter names / shapes;
-stored are the raw gradients of both steps, the statistics and the parameters after the second step."""
+stored are the raw gradients of both steps, the statistics and the parameters after the second step.  The first step's gradients
+are stored whole; of every hidden x hidden matrix, the second step's gradients and the final parameters keep a fixed sample of
+their entries (sample_large), which keeps the file under 1 MB."""
 import os
 import sys
 
@@ -20,6 +22,23 @@ CASES = [  # tag, state_dim, action_dim, continuous, hidden, layers, minibatch
     ("cont128", 3, (1,), True, 128, 2, 700),
     ("disc128x3", 4, 2, False, 128, 3, 500),
 ]
+SAMPLED = 2048      # entries kept of a sampled matrix
+
+
+def sample_large(out):
+    """For every parameter of more than 4 * SAMPLED entries, keep SAMPLED of them (`{tag}_sample_<name>`: sorted flat indices,
+    seed 0) in the second step's gradients and in the final parameters."""
+    rng = np.random.default_rng(0)
+    for tag, *_ in CASES:
+        for n in out[f"{tag}_names"]:
+            size = int(np.prod(out[f"{tag}_pshape_{n}"]))
+            if size <= 4 * SAMPLED:
+                continue
+            idx = np.sort(rng.choice(size, SAMPLED, replace=False)).astype(np.uint16 if size <= 1 << 16 else np.int64)
+            out[f"{tag}_sample_{n}"] = idx
+            for key in (f"{tag}_s1_g_{n}", f"{tag}_final_p_{n}"):
+                out[key] = out[key].reshape(-1)[idx]
+    return out
 
 
 def rollout_cases(ref_ac):
@@ -115,7 +134,7 @@ def main():
         for n, p in m.named_parameters():
             out[f"{tag}_final_p_{n}"] = p.detach().numpy().copy()
     path = os.path.join(OUT, "update_wide.npz")
-    np.savez_compressed(path, **out)
+    np.savez_compressed(path, **sample_large(out))
     print("wrote", path, os.path.getsize(path), "bytes")
 
 

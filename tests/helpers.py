@@ -27,6 +27,21 @@ def golden_policy(golden_dir, tag, file="model.npz", prefix="p"):
     return R.RefPolicy(named, continuous="actor_logstd" in names), named, g
 
 
+def golden_flat(g, tag, key, names):
+    """The golden arrays `{tag}_{key}_<name>` in flat_from_named order, and the mask of the full flat vector's entries they
+    hold: a parameter stored as a sample of its entries (`{tag}_sample_<name>`, sorted flat indices) gives only those."""
+    vals, mask = {}, {}
+    for n in names:
+        m = np.zeros(int(np.prod(g[f"{tag}_pshape_{n}"])), np.float32)
+        v = g[f"{tag}_{key}_{n}"]
+        if v.size == m.size:
+            m[:] = 1
+        else:
+            m[g[f"{tag}_sample_{n}"]] = 1
+        vals[n], mask[n] = v, m
+    return flat_from_named(vals), flat_from_named(mask).astype(bool)
+
+
 def random_policy(obs_dim, act_dim, hidden, num_layers, continuous, seed=0, scale=1.0):
     """Reference-shaped parameters with torch's default Linear init scale (deterministic)."""
     g = torch.Generator().manual_seed(seed)

@@ -76,3 +76,44 @@ def test_hidden_dim_flag_reaches_config_params_and_flop_count(monkeypatch):
     assert bench.workload_config("ppo", 1)["hidden_dim"] == 128 and bench.params("ppo", 1, 3)["hidden_dim"] == 128
     o, a = w["obs"], w["act"]
     assert bench.mlp_flops_fwd(w) == 2 * (o * 128 + 128 * 128 + 128 * a) + 2 * (o * 128 + 128 * 128 + 128) > 3 * f64
+
+
+def test_dump_outputs_writes_float_arrays_and_samples_large_ones(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    monkeypatch.setattr(bench, "DUMP_ELEMENTS", 100)
+    small, large = torch.arange(12, dtype=torch.int32).reshape(3, 4), torch.arange(1000, dtype=torch.float64)
+    bench.dump_outputs(str(tmp_path), {"small": small, "large": large})
+    s, l = np.load(tmp_path / "small.npy"), np.load(tmp_path / "large.npy")
+    assert s.dtype == np.float32 and np.array_equal(s, small.numpy())
+    assert l.dtype == np.float64 and l.shape == (100,) and np.all(np.diff(l) > 0)
+    assert np.array_equal(l, bench.seeded_sample(1000, 100).numpy())           # the same fixed sample every run
+    assert np.array_equal(bench.seeded_sample(5, 100).numpy(), np.arange(5))
+
+
+def test_dump_outputs_is_refused_for_the_reference_arm(tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=120)
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_timed_path(tmp_path):
+    """Two runs with the same arguments start from the same inputs: the dumped parameters and rollout agree."""
+    import numpy as np
+    runs = []
+    for k in range(2):
+        out = tmp_path / str(k)
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "3", "--no-cpu-baseline",
+                            "--no-extras", "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+        runs.append({p.stem: np.load(p) for p in out.glob("*.npy")})
+    a, b = runs
+    assert sorted(a) == ["actions", "advantages", "dones", "log_probs", "next_value", "obs", "params", "returns", "rewards", "stats",
+                         "values"]
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20 and all(v.dtype in (np.float32, np.float64) for v in a.values())
+    assert a["obs"].shape == (128, bench.DUMP_COLUMNS, 4) and a["stats"].shape == (16, 16)
+    assert np.isfinite(a["params"]).all() and np.isfinite(a["advantages"]).all()
+    np.testing.assert_allclose(a["params"], b["params"], rtol=1e-5, atol=1e-6)
+    np.testing.assert_allclose(a["returns"], b["returns"], rtol=1e-4, atol=1e-4)

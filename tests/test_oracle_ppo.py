@@ -110,7 +110,7 @@ def test_feistel_shuffle_restatement_is_a_permutation():
 def test_update_step_wide_shapes(golden_dir, tag):
     """The restated update against the reference's own gradients at 128 hidden units (tests/golden/update_wide.npz, written by
     oracle/gen_golden_wide.py from the imported reference): pins the checker of the wide GPU paths, not only the 64-wide one."""
-    from tests.helpers import flat_from_named
+    from tests.helpers import flat_from_named, golden_flat
     g = np.load(os.path.join(golden_dir, "update_wide.npz"))
     names = [str(n) for n in g[f"{tag}_names"]]
     named0 = {}
@@ -123,11 +123,11 @@ def test_update_step_wide_shapes(golden_dir, tag):
     t = lambda k: torch.from_numpy(g[f"{tag}_{k}"])
     for step in range(2):
         stats, raw, _, _ = R.ppo_update_step(pol, opt, t("obs"), t("act"), t("oldlp"), t("adv"), t("ret"), t("vold"), max_grad_norm=0.5)
-        want = flat_from_named({n: g[f"{tag}_s{step}_g_{n}"] for n in names})
-        got = flat_from_named({n: r.numpy() for n, r in zip(pol.p.keys(), raw)})
+        want, sel = golden_flat(g, tag, f"s{step}_g", names)
+        got = flat_from_named({n: r.numpy() for n, r in zip(pol.p.keys(), raw)})[sel]
         assert float(np.linalg.norm(got - want) / np.linalg.norm(want)) < 1e-6
         ref = g[f"{tag}_s{step}_stats"]
         np.testing.assert_allclose([stats[k] for k in ("policy_loss", "value_loss", "entropy", "loss", "old_approx_kl", "approx_kl", "clipfrac",
                                                        "grad_norm")], ref, rtol=2e-5, atol=1e-7)
-    np.testing.assert_allclose(flat_from_named({n: pol.p[n].detach().numpy() for n in names}),
-                               flat_from_named({n: g[f"{tag}_final_p_{n}"] for n in names}), rtol=1e-6, atol=1e-7)
+    want, sel = golden_flat(g, tag, "final_p", names)
+    np.testing.assert_allclose(flat_from_named({n: pol.p[n].detach().numpy() for n in names})[sel], want, rtol=1e-6, atol=1e-7)

@@ -7,7 +7,7 @@ import torch
 
 from aur_ppo_b200 import _lib, kernels
 from oracle import ppo_ref as R
-from tests.helpers import flat_from_named, random_policy
+from tests.helpers import flat_from_named, golden_flat, random_policy
 
 pytestmark = pytest.mark.gpu
 
@@ -131,11 +131,12 @@ def test_wide_update_matches_reference_golden(golden_dir, tag):
         grads = up.grad(*bufs, idx, clip_coeff=clip, entropy_coeff=ent_c, value_coeff=vf_c, norm_adv=True, clip_vloss=True).clone()
         assert L.aur_launch_count() >= 12                               # the layer-wise path, not the fused generic kernel
         stats = up.apply(lr, mgn).cpu().numpy()
-        want = flat_from_named({n: g[f"{tag}_s{step}_g_{n}"] for n in names})
-        got = grads[:up.P].cpu().numpy()
+        want, sel = golden_flat(g, tag, f"s{step}_g", names)
+        got = grads[:up.P].cpu().numpy()[sel]
         print(f"{tag} step {step}: rel L2 vs the reference's gradients {_rel_l2(got, want):.2e}")
         np.testing.assert_allclose(got, want, rtol=1e-4, atol=1e-4 * float(np.abs(want).max()) + 1e-9)
         assert _rel_l2(got, want) < 1e-4
         ref = g[f"{tag}_s{step}_stats"]
         np.testing.assert_allclose([stats[0], stats[1], stats[2], stats[7], stats[3], stats[4], stats[5], stats[6]], ref, rtol=1e-4, atol=2e-6)
-    np.testing.assert_allclose(params.cpu().numpy(), flat_from_named({n: g[f"{tag}_final_p_{n}"] for n in names}), rtol=1e-5, atol=1e-6)
+    want, sel = golden_flat(g, tag, "final_p", names)
+    np.testing.assert_allclose(params.cpu().numpy()[sel], want, rtol=1e-5, atol=1e-6)
