@@ -55,6 +55,22 @@ class UpdateArgs(ctypes.Structure):
                 ("rec_actor", c_void_p), ("rec_critic", c_void_p)]
 
 
+class PopDesc(ctypes.Structure):
+    _fields_ = [("K", c_int32), ("_pad", c_int32), ("n_member", c_int64), ("seeds", c_void_p)]
+
+
+class PopHparams(ctypes.Structure):
+    _fields_ = [("learning_rate", c_double), ("entropy_coeff", c_double), ("clip_coeff", c_double), ("value_coeff", c_double),
+                ("max_grad_norm", c_double), ("target_kl", c_double)]
+
+
+class PopUpdateArgs(ctypes.Structure):
+    _fields_ = [("policy", PolicyDesc), ("norm_adv", c_int32), ("clip_vloss", c_int32), ("mb_index", c_int32), ("n_mb", c_int32),
+                ("m", c_int64), ("idx", c_void_p), ("rec_actor", c_void_p), ("rec_critic", c_void_p), ("params", c_void_p),
+                ("hparams", c_void_p), ("adv_moments", c_void_p), ("active", c_void_p), ("workspace", c_void_p),
+                ("grads_out", c_void_p)]
+
+
 DP_MAX_RANKS = 16
 DP_HANDLE_BYTES = 64
 
@@ -243,6 +259,21 @@ def lib() -> ctypes.CDLL:
     L.aur_adam_flat.restype = c_int
     L.aur_adam_flat.argtypes = [c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_double, c_double, c_double, c_double,
                                 c_int64, c_void_p, c_double, c_void_p]
+    L.aur_pop_rollout.restype = c_int
+    L.aur_pop_rollout.argtypes = [ctypes.POINTER(PopDesc), ctypes.POINTER(RolloutArgs), c_void_p]
+    L.aur_pop_shuffle_indices.restype = c_int
+    L.aur_pop_shuffle_indices.argtypes = [ctypes.POINTER(PopDesc), c_int32, c_int32, c_uint64, c_void_p, c_void_p]
+    L.aur_pop_adv_moments_multi.restype = c_int
+    L.aur_pop_adv_moments_multi.argtypes = [ctypes.POINTER(PopDesc), c_int32, c_int64, c_void_p, c_void_p, c_void_p, c_void_p,
+                                            c_void_p]
+    L.aur_pop_update_workspace_bytes.restype = c_int64
+    L.aur_pop_update_workspace_bytes.argtypes = [ctypes.POINTER(PopDesc), ctypes.POINTER(PolicyDesc), c_int32, c_int64]
+    L.aur_pop_update_grad.restype = c_int
+    L.aur_pop_update_grad.argtypes = [ctypes.POINTER(PopDesc), ctypes.POINTER(PopUpdateArgs), c_void_p]
+    L.aur_pop_update_apply.restype = c_int
+    L.aur_pop_update_apply.argtypes = [ctypes.POINTER(PopDesc), ctypes.POINTER(PolicyDesc), c_void_p, c_void_p, c_void_p, c_void_p,
+                                       c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_double, c_double, c_double, c_double,
+                                       c_int64, c_void_p, c_int32, c_int32, c_int32, c_void_p]
     L.aur_sincos_f64.restype = c_int
     L.aur_sincos_f64.argtypes = [c_int64, c_void_p, c_void_p, c_void_p, c_void_p]
     _lib = L

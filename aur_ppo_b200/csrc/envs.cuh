@@ -322,6 +322,10 @@ struct RolloutDev {
   double gamma;
   int t0;                     // first step index of this launch (buffers / episode log); 0 except for the per-step launches of rollout_wide.cu
   const float* ext_logits;    // [N][4] actor outputs computed outside the kernel (rollout_tc_kernel<ENV, 0>), else nullptr
+  // populations (rollout_tc_kernel<ENV, H, true>, aur_pop_rollout): N = K * n_member columns, member k = blockIdx.y owns
+  // columns k * n_member ..; its parameters sit at params + k * pop_P, its Philox key is pop_seeds[k]
+  long long n_member, pop_P;
+  const uint64_t* pop_seeds;
 };
 
 template <int HID>

@@ -480,6 +480,7 @@ static aur::RolloutDev to_dev(const aur_rollout_args& a) {
   d.obs_buf = a.obs_buf; d.act_buf = a.act_buf; d.logp_buf = a.logp_buf; d.val_buf = a.val_buf; d.rew_buf = a.rew_buf;
   d.done_buf = a.done_buf; d.next_obs = a.next_obs; d.next_done = a.next_done; d.next_value = a.next_value;
   d.t0 = 0; d.ext_logits = nullptr;
+  d.n_member = 0; d.pop_P = 0; d.pop_seeds = nullptr;
   d.actions_in = a.actions_in; d.seed = a.seed; d.step0 = a.step0; d.env_id0 = a.env_id0; d.log = a.log; d.gamma = a.gamma;
   return d;
 }
@@ -583,6 +584,55 @@ extern "C" int aur_rollout(const aur_rollout_args* args, void* stream) {
     if ((rc = launch_critic_values_tc(critic, a.policy.obs_dim, 64, a.obs_buf, (long long)a.T * a.N, a.val_buf, s))) return rc;
     if (a.next_value && (rc = launch_critic_values_tc(critic, a.policy.obs_dim, 64, a.next_obs, a.N, a.next_value, s))) return rc;
   }
+  return 0;
+}
+
+namespace aur {
+int check_pop(const aur_pop_desc* pop, const char* who);                    // update.cu
+int check_pop_policy(const aur_policy_desc& p, const char* who);
+int launch_rollout_tc_pop(const RolloutDev& d, int env_kind, int K, cudaStream_t s);   // rollout_tc.cu
+int launch_critic_values_tc_pop(const float* critic, int obs_dim, const float* obs, long long segs, int K, long long n_member,
+                                long long P, float* out, cudaStream_t s);   // values_tc.cu
+}  // namespace aur
+
+extern "C" int aur_pop_rollout(const aur_pop_desc* pop, const aur_rollout_args* args, void* stream) {
+  using namespace aur;
+  int rc = check_pop(pop, "aur_pop_rollout");
+  if (rc) return rc;
+  if (!args) { set_error("aur_pop_rollout: null args"); return AUR_ERR_ARG; }
+  const aur_rollout_args& a = *args;
+  if ((rc = check_pop_policy(a.policy, "aur_pop_rollout"))) return rc;
+  const int ek = a.env_kind;
+  if (ek != AUR_ENV_CARTPOLE && ek != AUR_ENV_PENDULUM && ek != AUR_ENV_MOUNTAINCAR) {
+    set_error("aur_pop_rollout: env_kind %d has no population kernel (CartPole-v1, Pendulum-v1, MountainCar-v0); no fallback", ek);
+    return AUR_ERR_UNSUPPORTED;
+  }
+  const bool cont = ek == AUR_ENV_PENDULUM;
+  const int want_obs = ek == AUR_ENV_CARTPOLE ? 4 : (cont ? 3 : 2), want_act = ek == AUR_ENV_CARTPOLE ? 2 : (cont ? 1 : 3);
+  if ((a.policy.continuous != 0) != cont || a.policy.obs_dim != want_obs || a.policy.act_dim != want_act) {
+    set_error("aur_pop_rollout: env_kind %d needs obs %d, %d %s actions", ek, want_obs, want_act, cont ? "continuous" : "discrete");
+    return AUR_ERR_ARG;
+  }
+  if (a.T < 1 || a.N != (int64_t)pop->K * pop->n_member) {
+    set_error("aur_pop_rollout: need T >= 1 and N = K * n_member (got T %d, N %lld, K %d, n_member %lld)", a.T, (long long)a.N, pop->K,
+              (long long)pop->n_member);
+    return AUR_ERR_ARG;
+  }
+  if (!a.params || !a.obs_buf || !a.act_buf || !a.logp_buf || !a.val_buf || !a.rew_buf || !a.done_buf || !a.next_obs ||
+      !a.next_done || !a.env.phys || !a.env.pcg || !a.env.elapsed || !a.env.ep_return || !a.env.ep_length ||
+      (cont && a.wrappers && !a.env.norm) || a.log.entries || a.log.count) {
+    set_error("aur_pop_rollout: null buffer, wrappers without env.norm, or a full episode log (not supported for populations)");
+    return AUR_ERR_ARG;
+  }
+  RolloutDev d = to_dev(a);
+  d.n_member = pop->n_member; d.pop_seeds = pop->seeds; d.pop_P = policy_param_count(a.policy);
+  cudaStream_t s = (cudaStream_t)stream;
+  if ((rc = launch_rollout_tc_pop(d, ek, pop->K, s))) return rc;
+  const float* critic = a.params + net_param_count(a.policy.obs_dim, 64, 2, a.policy.act_dim);
+  if ((rc = launch_critic_values_tc_pop(critic, a.policy.obs_dim, a.obs_buf, a.T, pop->K, pop->n_member, d.pop_P, a.val_buf, s))) return rc;
+  if (a.next_value &&
+      (rc = launch_critic_values_tc_pop(critic, a.policy.obs_dim, a.next_obs, 1, pop->K, pop->n_member, d.pop_P, a.next_value, s)))
+    return rc;
   return 0;
 }
 

@@ -33,9 +33,13 @@ struct RtCfg {
 // H = 0: the actor's outputs come from outside (a.ext_logits [N][4], rollout_wide.cu computes them layer by layer for the widths
 // whose W2 does not fit shared memory); the kernel is then only the per-step env / sampling / bookkeeping part, launched once
 // per step (a.T = 1, a.t0 = step) with the env state round-tripping through its global arrays.
-template <class ENV, int H>
+// POP: population form (aur_pop_rollout), grid (ceil(n_member / 128), K): the CTA's member is blockIdx.y, its envs are the
+// member-local indices blockIdx.x * 128 + tid < n_member, stored in the population's columns k * n_member + local; the
+// weights, the Philox key and the episode-log row are the member's, the Philox counters and logged env ids member-local.
+template <class ENV, int H, bool POP = false>
 __global__ void __launch_bounds__(RT_S, RtCfg<H>::CTAS) rollout_tc_kernel(RolloutDev a) {
   using Cfg = RtCfg<H>;
+  static_assert(!POP || H == 64, "populations run the 64-wide kernel");
   constexpr bool EXT = H == 0;
   constexpr int KA = Cfg::KA;
   constexpr int RS_W1T = Cfg::S_W1T, RS_B1 = Cfg::S_B1, RS_B2 = Cfg::S_B2, RS_W3 = Cfg::S_W3, RS_B3 = Cfg::S_B3, RS_LS = Cfg::S_LS;
@@ -55,7 +59,7 @@ __global__ void __launch_bounds__(RT_S, RtCfg<H>::CTAS) rollout_tc_kernel(Rollou
   if (tid == 0) { mbar_init(bar, 1); mbar_fence_init(); }
   if (warp == 0) tc::tmem_alloc(tslot, H);
   {
-    const float* g = a.params;                    // the actor comes first in the flat buffer
+    const float* g = POP ? a.params + (long long)blockIdx.y * a.pop_P : a.params;   // the actor comes first in the flat buffer
     const float* gb1 = g + H * obs_dim;
     const float* gW2 = gb1 + H;
     const float* gb2 = gW2 + H * H;
@@ -70,7 +74,7 @@ __global__ void __launch_bounds__(RT_S, RtCfg<H>::CTAS) rollout_tc_kernel(Rollou
     if (tid < 4) {
       sw[RS_B3 + tid] = tid < A ? gb3[tid] : 0.0f;
       const int64_t gA = net_param_count(obs_dim, H, 2, A), gC = net_param_count(obs_dim, H, 2, 1);
-      sw[RS_LS + tid] = (a.continuous && tid < A) ? a.params[gA + gC + tid] : 0.0f;
+      sw[RS_LS + tid] = (a.continuous && tid < A) ? g[gA + gC + tid] : 0.0f;
     }
 #pragma unroll 1
     for (int e = tid; e < H * (H / 8); e += RT_S) {         // W2 row j, 8-feature chunk ch -> K atom ch / 8
@@ -91,8 +95,9 @@ __global__ void __launch_bounds__(RT_S, RtCfg<H>::CTAS) rollout_tc_kernel(Rollou
   constexpr uint32_t ID_FWD = tc::instr_desc(tc::FMT_BF16, 128, H, 0, 0);
 
   const long long N = a.N;
-  const long long n = (long long)blockIdx.x * RT_S + tid;
-  const bool live = n < N;
+  const long long n_loc = (long long)blockIdx.x * RT_S + tid;         // member-local env index (POP), else the column
+  const long long n = POP ? (long long)blockIdx.y * a.n_member + n_loc : n_loc;
+  const bool live = POP ? n_loc < a.n_member : n < N;
   const long long m0 = live ? n : 0;
   ENV env;
   NormState nm;
@@ -160,12 +165,14 @@ __global__ void __launch_bounds__(RT_S, RtCfg<H>::CTAS) rollout_tc_kernel(Rollou
     }
     }
     // the step's random numbers do not depend on the logits: draw them while the MMAs run
-    const uint64_t gid = a.env_id0 + (uint64_t)n, gstep = a.step0 + (uint64_t)t;
+    const uint64_t gid = a.env_id0 + (uint64_t)(POP ? n_loc : n), gstep = a.step0 + (uint64_t)t;
     Philox rnd;
     rnd.c[0] = rnd.c[1] = rnd.c[2] = rnd.c[3] = 0u;
-    if (a.actions_in == nullptr)
-      rnd = philox4x32_10((uint32_t)gid, (uint32_t)(gid >> 32), (uint32_t)gstep, (uint32_t)(gstep >> 32), (uint32_t)a.seed,
-                          (uint32_t)(a.seed >> 32));
+    if (a.actions_in == nullptr) {
+      const uint64_t seed = POP ? a.pop_seeds[blockIdx.y] : a.seed;
+      rnd = philox4x32_10((uint32_t)gid, (uint32_t)(gid >> 32), (uint32_t)gstep, (uint32_t)(gstep >> 32), (uint32_t)seed,
+                          (uint32_t)(seed >> 32));
+    }
     float head[POL_OUT_MAX];
     if constexpr (EXT) {
       const float4 lg = live ? __ldg(reinterpret_cast<const float4*>(a.ext_logits) + n) : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -253,7 +260,14 @@ __global__ void __launch_bounds__(RT_S, RtCfg<H>::CTAS) rollout_tc_kernel(Rollou
     a.rew_buf[o] = reward32;
     if (finished) {
       // ---- SyncVectorEnv autoreset: the returned obs is the RESET obs; `done` keeps `terminated`
-      log_episode(a.log, t, n, (int)gstep, (int)gid, ep_ret, ep_len);
+      if constexpr (POP) {                           // the member's row of the episode log, member-local env index
+        aur_episode_log lg = a.log;
+        if (lg.first_finished) lg.first_finished += (size_t)blockIdx.y * a.T;
+        if (lg.totals) lg.totals += 3 * (size_t)blockIdx.y;
+        log_episode(lg, t, n_loc, (int)gstep, (int)gid, ep_ret, ep_len);
+      } else {
+        log_episode(a.log, t, n, (int)gstep, (int)gid, ep_ret, ep_len);
+      }
       env.reset(rng);
       elapsed = 0; ep_ret = 0.0f; ep_len = 0;
       if constexpr (PEND) {
@@ -295,10 +309,29 @@ int rollout_impl() {
 }
 void set_rollout_impl(int impl) { g_rollout_impl = impl; }
 
-template <class ENV, int H>
+template <class ENV, int H, bool POP = false>
 static int rollout_tc_attrs() {
-  AUR_CUDA_OK(cudaFuncSetAttribute(rollout_tc_kernel<ENV, H>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RtCfg<H>::SMEM));
-  AUR_CUDA_OK(cudaFuncSetAttribute(rollout_tc_kernel<ENV, H>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  AUR_CUDA_OK(cudaFuncSetAttribute(rollout_tc_kernel<ENV, H, POP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RtCfg<H>::SMEM));
+  AUR_CUDA_OK(cudaFuncSetAttribute(rollout_tc_kernel<ENV, H, POP>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  return 0;
+}
+
+// population rollout (aur_pop_rollout): every member's envs in one launch, grid (ceil(n_member / 128), K)
+int launch_rollout_tc_pop(const RolloutDev& d, int env_kind, int K, cudaStream_t s) {
+  static DeviceOnce attr;
+  if (attr.first()) {
+    int rc;
+    if ((rc = rollout_tc_attrs<CartPole, 64, true>()) || (rc = rollout_tc_attrs<Pendulum, 64, true>()) ||
+        (rc = rollout_tc_attrs<MountainCar, 64, true>()))
+      return rc;
+    attr.done();
+  }
+  const dim3 grid((unsigned)((d.n_member + RT_S - 1) / RT_S), (unsigned)K);
+  constexpr size_t SM = RtCfg<64>::SMEM;
+  if (env_kind == AUR_ENV_PENDULUM) rollout_tc_kernel<Pendulum, 64, true><<<grid, RT_S, SM, s>>>(d);
+  else if (env_kind == AUR_ENV_MOUNTAINCAR) rollout_tc_kernel<MountainCar, 64, true><<<grid, RT_S, SM, s>>>(d);
+  else rollout_tc_kernel<CartPole, 64, true><<<grid, RT_S, SM, s>>>(d);
+  AUR_LAUNCH_OK("rollout_tc_kernel (population)");
   return 0;
 }
 

@@ -40,6 +40,29 @@ __global__ void __launch_bounds__(256) shuffle_kernel(long long n, int wa, int w
   out[i] = (int32_t)x;
 }
 
+// Population form (aur_pop_shuffle_indices): grid (ceil(n / 256), K, epochs); member k's epoch e is the permutation of
+// aur_shuffle_indices(n, seeds[k], stream_id0 + e), its round keys derived here (one Philox call per round, as the host does
+// for a single run), each local index j written as the population's global row.
+__global__ void __launch_bounds__(256) pop_shuffle_kernel(long long n, int wa, int wb, const uint64_t* __restrict__ seeds,
+                                                        uint64_t stream_id0, long long n_member, long long NK,
+                                                        int32_t* __restrict__ out) {
+  __shared__ ShufKeys keys;
+  const int k = blockIdx.y, e = blockIdx.z;
+  if (threadIdx.x < SHUF_ROUNDS) {
+    const uint64_t seed = seeds[k], stream_id = stream_id0 + (uint64_t)e;
+    keys.k[threadIdx.x] = philox4x32_10((uint32_t)threadIdx.x, (uint32_t)stream_id, (uint32_t)(stream_id >> 32), 0x5AFE5EEDu,
+                                        (uint32_t)seed, (uint32_t)(seed >> 32)).c[0];
+  }
+  __syncthreads();
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const ShufKeys kk = keys;
+  uint32_t x = (uint32_t)i;
+  do { x = shuf_encrypt(x, wa, wb, kk); } while ((long long)x >= n);
+  const long long t = (long long)x / n_member;
+  out[((long long)k * gridDim.z + e) * n + i] = (int32_t)(t * NK + (long long)k * n_member + ((long long)x - t * n_member));
+}
+
 // Packed per-sample records for the minibatch gather: the update reads ONE 32-byte sector per sample and net instead
 // of one sector per gathered array (4-byte elements at random rows cost 32 B of DRAM traffic each).
 //   actor  record: obs[0..3] (zero padded) | action[0], old logprob, advantage, action[1]
@@ -96,5 +119,26 @@ extern "C" int aur_shuffle_indices(int64_t n, uint64_t seed, uint64_t stream_id,
                               (uint32_t)(seed >> 32)).c[0];
   shuffle_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>((long long)n, wa, wb, keys, out);
   AUR_LAUNCH_OK("shuffle_kernel");
+  return 0;
+}
+
+extern "C" int aur_pop_shuffle_indices(const aur_pop_desc* pop, int32_t T, int32_t epochs, uint64_t stream_id0, int32_t* out,
+                                       void* stream) {
+  using namespace aur;
+  if (!pop || pop->K < 1 || pop->n_member < 1 || !pop->seeds || T < 1 || epochs < 1 || !out) {
+    set_error("aur_pop_shuffle_indices: bad arguments"); return AUR_ERR_ARG;
+  }
+  const long long n = (long long)T * pop->n_member, NK = (long long)pop->K * pop->n_member;
+  if ((long long)T * NK > 0x7FFFFFFFLL || pop->K > 65535 || epochs > 65535) {
+    set_error("aur_pop_shuffle_indices: K * T * n_member must be < 2^31 (got K %d, T %d, n_member %lld)", pop->K, T,
+              (long long)pop->n_member);
+    return AUR_ERR_ARG;
+  }
+  int bits = 1;
+  while ((1LL << bits) < n) ++bits;
+  const int wa = (bits + 1) / 2, wb = bits - wa > 0 ? bits - wa : 0;
+  pop_shuffle_kernel<<<dim3((unsigned)((n + 255) / 256), (unsigned)pop->K, (unsigned)epochs), 256, 0, (cudaStream_t)stream>>>(
+      n, wa, wb, pop->seeds, stream_id0, (long long)pop->n_member, NK, out);
+  AUR_LAUNCH_OK("pop_shuffle_kernel");
   return 0;
 }

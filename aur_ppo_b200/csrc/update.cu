@@ -434,10 +434,25 @@ __global__ void __launch_bounds__(UPD_THREADS, 1) ppo_grad_kernel(UpdDev a) {
   }
 }
 
+// Population form of the reduction (grid.y = K): member k's ncta real partial rows at partials + k * part_stride, summed with
+// the quarter boundaries of the single run's chunk_ncta rows (the rows a single run has beyond ncta are the exact zeros its
+// idle CTAs write), into grads_out + k * grads_stride; inactive members are skipped.
+struct PopRed {
+  int chunk_ncta;
+  long long part_stride, grads_stride;
+  const int32_t* active;
+};
+
 // grads_out[p] = sum over CTAs of the partials, in CTA order, fp64 accumulation.
+template <bool POP = false>
 __global__ void grad_reduce_kernel(const float* __restrict__ partials, int ncta, int obs_dim, int act_dim, int continuous,
                                    int hidden, int nl, int pstride, float* __restrict__ grads_out, DpDev dp,
-                                   unsigned int* __restrict__ ticket) {
+                                   unsigned int* __restrict__ ticket, PopRed pop) {
+  if constexpr (POP) {
+    if (!pop.active[blockIdx.y]) return;
+    partials += blockIdx.y * pop.part_stride;
+    grads_out += blockIdx.y * pop.grads_stride;
+  }
   const int64_t nA = net_param_count(obs_dim, hidden, nl, act_dim), nC = net_param_count(obs_dim, hidden, nl, 1);
   const int64_t P = nA + nC + (continuous ? act_dim : 0);
   // four lanes per output: lane q sums its quarter of the CTA partials in CTA order (fp64), the quarters are combined as
@@ -461,7 +476,7 @@ __global__ void grad_reduce_kernel(const float* __restrict__ partials, int ncta,
     }
     if (!zero) {
       const float* p = partials + (size_t)net * ncta * pstride + off;
-      const int chunk = (ncta + 3) >> 2;
+      const int chunk = ((POP ? pop.chunk_ncta : ncta) + 3) >> 2;
       int c = q * chunk;
       const int c1 = min(ncta, c + chunk);
       for (; c + 8 <= c1; c += 8) {                     // 8 loads in flight
@@ -571,14 +586,18 @@ __global__ void __launch_bounds__(256) adv_moments_kernel(long long m, const int
 // The same for all n_mb minibatches of an iteration at once: grid = (CTAs per minibatch, n_mb).  The last CTA of a minibatch
 // finalises it (fixed order) and, data-parallel, pushes its three moments to every rank; the last minibatch to finish
 // releases the flags - ONE rendezvous per iteration instead of one per minibatch.
+// POP (aur_pop_adv_moments_multi): grid (cpm, n_mb, K), entry (k, y) = index list k * n_mb + y; the CTAs only write their
+// partials, pop_moments_final_kernel combines them in the order of the last-CTA finalisation below.
+template <bool POP = false>
 __global__ void __launch_bounds__(256) adv_moments_multi_kernel(long long m, const int32_t* __restrict__ idx, long long idx_stride,
                                                               const float* __restrict__ adv, double* __restrict__ partial,
                                                               unsigned int* __restrict__ tickets, double* __restrict__ out, DpDev dp) {
   __shared__ double sh[2][8];
   __shared__ bool last, last_of_all;
   const int y = blockIdx.y;
-  const int32_t* my_idx = idx ? idx + (long long)y * idx_stride : nullptr;
-  const long long row0 = (long long)y * idx_stride;
+  const long long entry = POP ? (long long)blockIdx.z * gridDim.y + y : y;
+  const int32_t* my_idx = idx ? idx + entry * idx_stride : nullptr;
+  const long long row0 = entry * idx_stride;
   double s = 0.0, ss = 0.0;
   const long long stride = (long long)gridDim.x * blockDim.x;
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -600,15 +619,18 @@ __global__ void __launch_bounds__(256) adv_moments_multi_kernel(long long m, con
   s = warp_sum(s); ss = warp_sum(ss);
   if ((threadIdx.x & 31) == 0) { sh[0][threadIdx.x >> 5] = s; sh[1][threadIdx.x >> 5] = ss; }
   __syncthreads();
-  double* part = partial + (size_t)y * gridDim.x * 2;
+  double* part = partial + (size_t)entry * gridDim.x * 2;
   if (threadIdx.x == 0) {
     double a = 0.0, b = 0.0;
     for (int w = 0; w < 8; ++w) { a += sh[0][w]; b += sh[1][w]; }
     part[2 * blockIdx.x] = a; part[2 * blockIdx.x + 1] = b;
-    __threadfence();
-    last = atomicAdd(tickets + 1 + y, 1u) == gridDim.x - 1;
-    last_of_all = false;
+    if constexpr (!POP) {
+      __threadfence();
+      last = atomicAdd(tickets + 1 + y, 1u) == gridDim.x - 1;
+      last_of_all = false;
+    }
   }
+  if constexpr (POP) return;                             // the whole CTA: pop_moments_final_kernel finalises
   __syncthreads();
   if (!last) return;
   __threadfence();
@@ -636,39 +658,26 @@ __global__ void __launch_bounds__(256) adv_moments_multi_kernel(long long m, con
   }
 }
 
-// clip_grad_norm_ (all parameters, torch semantics) + Adam, one CTA (P ~ 9e3).
-__global__ void __launch_bounds__(1024) adam_kernel(int64_t P, float* __restrict__ params, float* __restrict__ g_in,
-                                                   float* __restrict__ m1, float* __restrict__ m2, float lr_over_bc1,
-                                                   float beta1, float beta2, float eps, float sqrt_bc2, float max_norm,
-                                                   float inv_m, float ent_c, float vf_c, float* __restrict__ stats_out, DpDev dp) {
+// the finalisation of adv_moments_multi_kernel<true>: entry e = (member, minibatch) sums its cpm CTA partials in CTA order
+__global__ void __launch_bounds__(128) pop_moments_final_kernel(int entries, int cpm, long long m, const double* __restrict__ partial,
+                                                              double* __restrict__ out) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= entries) return;
+  const double* part = partial + (size_t)e * cpm * 2;
+  double a = 0.0, b = 0.0;
+  for (int c = 0; c < cpm; ++c) { a += __ldcg(part + 2 * c); b += __ldcg(part + 2 * c + 1); }
+  out[3 * e] = a; out[3 * e + 1] = b; out[3 * e + 2] = (double)m;
+}
+
+// clip_grad_norm_ (all parameters, torch semantics) + Adam on one flat buffer by one CTA: the part of adam_kernel after the
+// data-parallel gather, shared with pop_adam_kernel
+__device__ __forceinline__ void adam_clip_step(int64_t P, float* __restrict__ params, const float* __restrict__ g_in,
+                                               float* __restrict__ m1, float* __restrict__ m2, float lr_over_bc1, float beta1,
+                                               float beta2, float eps, float sqrt_bc2, float max_norm, float inv_m, float ent_c,
+                                               float vf_c, float* __restrict__ stats_out) {
   __shared__ double sh[32];
   __shared__ float coef_s, norm_s;
   double ss = 0.0;
-  if (dp.world > 1) {
-    // data-parallel: the all-reduce happens HERE.  Every rank pushed its [grads | stats] sums into our exchange
-    // area (grad_reduce_kernel); wait for the flags, add the G vectors in rank order (bit-identical on every
-    // rank), keep the global sums in g_in, then clip + Adam as usual on replicated parameters.
-    unsigned char* me = dp.peer[dp.rank];
-    const uint64_t t_in = global_timer_ns();
-    if ((int)threadIdx.x < dp.world) dp_wait_flag(reinterpret_cast<const uint32_t*>(me + DP_OFF_FLAG_GRAD) + threadIdx.x, dp.seq, me);
-    __syncthreads();
-    if (threadIdx.x == 0) {                              // wall time this rank stood still waiting for the slowest peer
-      unsigned long long* w = reinterpret_cast<unsigned long long*>(me + DP_OFF_WAIT) + 4;
-      w[0] += (unsigned long long)(global_timer_ns() - t_in);
-      w[1] += 1ull;
-    }
-    // a wait gave up (a peer is gone): the sums are incomplete - do NOT step the parameters on them; the status word stays set
-    // and the host raises on every rank (ppo.train checks it once per update)
-    if (*reinterpret_cast<volatile uint32_t*>(me + DP_OFF_STATUS) != 0u) return;
-    const int gs = dp_grad_stride(P);
-    const float* rg = reinterpret_cast<const float*>(me + DP_OFF_GRAD) + (size_t)(dp.seq & 1u) * DP_MAX * gs;
-    for (int64_t i = threadIdx.x; i < P + AUR_NUM_STATS; i += blockDim.x) {
-      float g = 0.0f;
-      for (int r = 0; r < dp.world; ++r) g += __ldcg(rg + (size_t)r * gs + i);
-      g_in[i] = g;
-    }
-    __syncthreads();
-  }
   for (int64_t i = threadIdx.x; i < P; i += blockDim.x) { const double g = g_in[i]; ss += g * g; }
   ss = warp_sum(ss);
   if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = ss;
@@ -700,6 +709,75 @@ __global__ void __launch_bounds__(1024) adam_kernel(int64_t P, float* __restrict
     if (threadIdx.x == AUR_STAT_LOSS)
       v = st[AUR_STAT_POLICY_LOSS] * inv_m - ent_c * (st[AUR_STAT_ENTROPY] * inv_m) + (st[AUR_STAT_VALUE_LOSS] * inv_m) * vf_c;
     stats_out[threadIdx.x] = v;
+  }
+}
+
+// clip_grad_norm_ (all parameters, torch semantics) + Adam, one CTA (P ~ 9e3).
+__global__ void __launch_bounds__(1024) adam_kernel(int64_t P, float* __restrict__ params, float* __restrict__ g_in,
+                                                   float* __restrict__ m1, float* __restrict__ m2, float lr_over_bc1,
+                                                   float beta1, float beta2, float eps, float sqrt_bc2, float max_norm,
+                                                   float inv_m, float ent_c, float vf_c, float* __restrict__ stats_out, DpDev dp) {
+  if (dp.world > 1) {
+    // data-parallel: the all-reduce happens HERE.  Every rank pushed its [grads | stats] sums into our exchange
+    // area (grad_reduce_kernel); wait for the flags, add the G vectors in rank order (bit-identical on every
+    // rank), keep the global sums in g_in, then clip + Adam as usual on replicated parameters.
+    unsigned char* me = dp.peer[dp.rank];
+    const uint64_t t_in = global_timer_ns();
+    if ((int)threadIdx.x < dp.world) dp_wait_flag(reinterpret_cast<const uint32_t*>(me + DP_OFF_FLAG_GRAD) + threadIdx.x, dp.seq, me);
+    __syncthreads();
+    if (threadIdx.x == 0) {                              // wall time this rank stood still waiting for the slowest peer
+      unsigned long long* w = reinterpret_cast<unsigned long long*>(me + DP_OFF_WAIT) + 4;
+      w[0] += (unsigned long long)(global_timer_ns() - t_in);
+      w[1] += 1ull;
+    }
+    // a wait gave up (a peer is gone): the sums are incomplete - do NOT step the parameters on them; the status word stays set
+    // and the host raises on every rank (ppo.train checks it once per update)
+    if (*reinterpret_cast<volatile uint32_t*>(me + DP_OFF_STATUS) != 0u) return;
+    const int gs = dp_grad_stride(P);
+    const float* rg = reinterpret_cast<const float*>(me + DP_OFF_GRAD) + (size_t)(dp.seq & 1u) * DP_MAX * gs;
+    for (int64_t i = threadIdx.x; i < P + AUR_NUM_STATS; i += blockDim.x) {
+      float g = 0.0f;
+      for (int r = 0; r < dp.world; ++r) g += __ldcg(rg + (size_t)r * gs + i);
+      g_in[i] = g;
+    }
+    __syncthreads();
+  }
+  adam_clip_step(P, params, g_in, m1, m2, lr_over_bc1, beta1, beta2, eps, sqrt_bc2, max_norm, inv_m, ent_c, vf_c, stats_out);
+}
+
+// Population clip + Adam (aur_pop_update_apply): one CTA per member with the member's learning rate, step count, bias
+// corrections (host table) and coefficients; at the end of an epoch a member over its target_kl leaves `active`.
+struct PopAdam {
+  int64_t P;
+  float* params;
+  const float* grads;
+  float *m1, *m2;
+  int64_t* steps;
+  int32_t* active;
+  const aur_pop_hparams* hp;
+  const double* bc;
+  int64_t bc_len;
+  double frac;
+  float beta1, beta2, eps, inv_m;
+  float* stats;
+  int stats_rows, stats_row, epoch_end;
+};
+__global__ void __launch_bounds__(1024) pop_adam_kernel(PopAdam a) {
+  const int k = blockIdx.x;
+  if (!a.active[k]) return;
+  const int64_t step = a.steps[k] + 1;
+  if (step >= a.bc_len) return;                        // the host sizes the table for every step of the run
+  const aur_pop_hparams h = a.hp[k];
+  const double lr = h.learning_rate * a.frac;          // ppo.run_update: frac * learning_rate (1.0 without the anneal)
+  const double bc1 = a.bc[2 * step], bc2 = a.bc[2 * step + 1];
+  const float* g = a.grads + (size_t)k * (a.P + AUR_NUM_STATS);
+  float* st = a.stats ? a.stats + ((size_t)k * a.stats_rows + a.stats_row) * AUR_NUM_STATS : nullptr;
+  adam_clip_step(a.P, a.params + (size_t)k * a.P, g, a.m1 + (size_t)k * a.P, a.m2 + (size_t)k * a.P, (float)(lr / bc1), a.beta1,
+                 a.beta2, a.eps, (float)sqrt(bc2), (float)h.max_grad_norm, a.inv_m, (float)h.entropy_coeff, (float)h.value_coeff, st);
+  if (threadIdx.x == 0) {
+    a.steps[k] = step;
+    // ppo.py:271-273 on the value the stats row holds (fp32, compared in double as `stats_rows[n - 1, 4].item() > target_kl`)
+    if (a.epoch_end && (double)(g[a.P + AUR_STAT_APPROX_KL] * a.inv_m) > h.target_kl) a.active[k] = 0;
   }
 }
 
@@ -900,7 +978,7 @@ extern "C" int aur_ppo_update_grad(const aur_update_args* args, void* stream) {
   ticket2 += 1;
   grad_reduce_kernel<<<(4 * total + 255) / 256, 256, 0, s>>>(partials, gx, u.policy.obs_dim, u.policy.act_dim, u.policy.continuous,
                                                         u.policy.hidden_dim, u.policy.num_layers, pstride, u.grads_out, d.dp,
-                                                        ticket2);
+                                                        ticket2, PopRed{});
   AUR_LAUNCH_OK("grad_reduce_kernel");
   return 0;
 }
@@ -930,5 +1008,132 @@ extern "C" int aur_ppo_update_apply_dp(const aur_policy_desc* desc, float* param
                                                    (float)(1.0 / (double)m_total), (float)entropy_coeff, (float)value_coeff,
                                                    stats_out, dpd);
   AUR_LAUNCH_OK("adam_kernel");
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------ populations
+namespace aur {
+int check_pop(const aur_pop_desc* pop, const char* who) {
+  if (!pop || pop->K < 1 || pop->K > 65535 || pop->n_member < 1 || !pop->seeds) {
+    set_error("%s: bad population (need 1 <= K <= 65535, n_member >= 1, a device seed array)", who); return AUR_ERR_ARG;
+  }
+  return 0;
+}
+int check_pop_policy(const aur_policy_desc& p, const char* who) {
+  if (!is_headline_shape(p) || (p.continuous && p.act_dim > 2)) {
+    set_error("%s: populations run the 64 x 2 tensor-core kernels (hidden 64, 2 layers, obs_dim <= 4, act_dim <= 4, <= 2 continuous "
+              "dims); got hidden %d, %d layers, obs %d, act %d - no fallback", who, p.hidden_dim, p.num_layers, p.obs_dim, p.act_dim);
+    return AUR_ERR_UNSUPPORTED;
+  }
+  return 0;
+}
+// CTAs per net and member: a single run's count (#SM), or fewer when the member's minibatch has fewer tiles of 128 samples
+static int pop_grad_ctas(int64_t m) {
+  const int64_t tiles = (m + 127) / 128;
+  return (int)(tiles < sm_count() ? tiles : sm_count());
+}
+// CTAs per minibatch of the advantage moments: as aur_ppo_adv_moments_multi computes it
+static int pop_moment_ctas(int32_t n_mb, int64_t m) {
+  int cpm = MOM_CTAS / n_mb;
+  if (cpm < 1) cpm = 1;
+  const long long need = (m + 255) / 256;
+  if (cpm > need) cpm = (int)need;
+  return cpm;
+}
+static size_t pop_grad_ws_floats(int K, int64_t m) { return (size_t)K * 2 * pop_grad_ctas(m) * UPD_PSTRIDE; }
+}  // namespace aur
+
+extern "C" int64_t aur_pop_update_workspace_bytes(const aur_pop_desc* pop, const aur_policy_desc* desc, int32_t n_mb, int64_t m) {
+  using namespace aur;
+  int rc = check_pop(pop, "aur_pop_update_workspace_bytes");
+  if (rc) return rc;
+  if (!desc) { set_error("aur_pop_update_workspace_bytes: null policy"); return AUR_ERR_ARG; }
+  if ((rc = check_pop_policy(*desc, "aur_pop_update_workspace_bytes"))) return rc;
+  if (n_mb < 1 || n_mb > DP_MAXMB || m < 1) { set_error("aur_pop_update_workspace_bytes: need 1 <= n_mb <= %d, m >= 1", DP_MAXMB); return AUR_ERR_ARG; }
+  // [K][2][c][PSTRIDE] gradient partials | [K][n_mb][cpm][2] fp64 moment partials
+  return (int64_t)(pop_grad_ws_floats(pop->K, m) * sizeof(float) + (size_t)pop->K * n_mb * pop_moment_ctas(n_mb, m) * 2 * sizeof(double));
+}
+
+extern "C" int aur_pop_adv_moments_multi(const aur_pop_desc* pop, int32_t n_mb, int64_t m, const int32_t* idx, const float* advantages,
+                                         double* moments_out, float* workspace, void* stream) {
+  using namespace aur;
+  int rc = check_pop(pop, "aur_pop_adv_moments_multi");
+  if (rc) return rc;
+  if (n_mb <= 0 || n_mb > DP_MAXMB || m <= 0 || !idx || !advantages || !moments_out || !workspace) {
+    set_error("aur_pop_adv_moments_multi: bad arguments (1 <= n_mb <= %d, m >= 1, non-null arrays)", DP_MAXMB); return AUR_ERR_ARG;
+  }
+  const int cpm = pop_moment_ctas(n_mb, m);
+  double* partial = reinterpret_cast<double*>(workspace + pop_grad_ws_floats(pop->K, m));
+  DpDev dpd;
+  make_dp(nullptr, 1u, dpd, "aur_pop_adv_moments_multi");
+  cudaStream_t s = (cudaStream_t)stream;
+  adv_moments_multi_kernel<true><<<dim3((unsigned)cpm, (unsigned)n_mb, (unsigned)pop->K), 256, 0, s>>>(
+      (long long)m, idx, (long long)m, advantages, partial, nullptr, moments_out, dpd);
+  AUR_LAUNCH_OK("adv_moments_multi_kernel (population)");
+  const int entries = pop->K * n_mb;
+  pop_moments_final_kernel<<<(entries + 127) / 128, 128, 0, s>>>(entries, cpm, (long long)m, partial, moments_out);
+  AUR_LAUNCH_OK("pop_moments_final_kernel");
+  return 0;
+}
+
+extern "C" int aur_pop_update_grad(const aur_pop_desc* pop, const aur_pop_update_args* args, void* stream) {
+  using namespace aur;
+  int rc = check_pop(pop, "aur_pop_update_grad");
+  if (rc) return rc;
+  if (!args) { set_error("aur_pop_update_grad: null args"); return AUR_ERR_ARG; }
+  const aur_pop_update_args& u = *args;
+  if ((rc = check_pop_policy(u.policy, "aur_pop_update_grad"))) return rc;
+  if (u.m < 1 || u.n_mb < 1 || u.n_mb > DP_MAXMB || u.mb_index < 0 || u.mb_index >= u.n_mb || !u.idx || !u.rec_actor || !u.rec_critic ||
+      !u.params || !u.hparams || !u.active || !u.workspace || !u.grads_out || (u.norm_adv && !u.adv_moments) ||
+      ((uintptr_t)u.rec_actor & 31) || ((uintptr_t)u.rec_critic & 31)) {
+    set_error("aur_pop_update_grad: bad arguments"); return AUR_ERR_ARG;
+  }
+  const int64_t P = policy_param_count(u.policy);
+  UpdDev d{};
+  d.m_local = u.m; d.idx = u.idx + (size_t)u.mb_index * u.m; d.idx_offset = 0;
+  d.params = u.params;
+  d.obs_dim = u.policy.obs_dim; d.act_dim = u.policy.act_dim; d.continuous = u.policy.continuous;
+  d.norm_adv = u.norm_adv; d.clip_vloss = u.clip_vloss;
+  d.inv_m = (float)(1.0 / (double)u.m);
+  d.moments = u.norm_adv ? u.adv_moments + 3 * (size_t)u.mb_index : nullptr;
+  d.partials = u.workspace;
+  make_dp(nullptr, 0u, d.dp, "aur_pop_update_grad");
+  d.rec_actor = reinterpret_cast<const float4*>(u.rec_actor); d.rec_critic = reinterpret_cast<const float4*>(u.rec_critic);
+  const int gx = pop_grad_ctas(u.m);
+  PopUpd pu;
+  pu.hp = u.hparams; pu.active = u.active; pu.P = P;
+  pu.idx_stride = (long long)u.n_mb * u.m; pu.mom_stride = 3LL * u.n_mb; pu.part_stride = 2LL * gx * UPD_PSTRIDE;
+  cudaStream_t s = (cudaStream_t)stream;
+  if ((rc = launch_ppo_grad_tc_pop(d, pu, gx, pop->K, s))) return rc;
+  PopRed pr;
+  pr.chunk_ncta = sm_count(); pr.part_stride = pu.part_stride; pr.grads_stride = P + AUR_NUM_STATS; pr.active = u.active;
+  const int total = (int)(P + AUR_NUM_STATS);
+  grad_reduce_kernel<true><<<dim3((4 * total + 255) / 256, pop->K), 256, 0, s>>>(
+      u.workspace, gx, u.policy.obs_dim, u.policy.act_dim, u.policy.continuous, u.policy.hidden_dim, u.policy.num_layers, UPD_PSTRIDE,
+      u.grads_out, d.dp, nullptr, pr);
+  AUR_LAUNCH_OK("grad_reduce_kernel (population)");
+  return 0;
+}
+
+extern "C" int aur_pop_update_apply(const aur_pop_desc* pop, const aur_policy_desc* desc, const aur_pop_hparams* hparams, float* params,
+                                    const float* grads, float* adam_m, float* adam_v, int64_t* steps, int32_t* active, const double* bc,
+                                    int64_t bc_len, double frac, double beta1, double beta2, double eps, int64_t m_total,
+                                    float* stats_out, int32_t stats_rows, int32_t stats_row, int32_t epoch_end, void* stream) {
+  using namespace aur;
+  int rc = check_pop(pop, "aur_pop_update_apply");
+  if (rc) return rc;
+  if (!desc || !hparams || !params || !grads || !adam_m || !adam_v || !steps || !active || !bc || bc_len < 2 || m_total <= 0 ||
+      (stats_out && (stats_rows < 1 || stats_row < 0 || stats_row >= stats_rows))) {
+    set_error("aur_pop_update_apply: bad arguments"); return AUR_ERR_ARG;
+  }
+  if ((rc = check_pop_policy(*desc, "aur_pop_update_apply"))) return rc;
+  PopAdam a;
+  a.P = policy_param_count(*desc);
+  a.params = params; a.grads = grads; a.m1 = adam_m; a.m2 = adam_v; a.steps = steps; a.active = active; a.hp = hparams;
+  a.bc = bc; a.bc_len = bc_len; a.frac = frac;
+  a.beta1 = (float)beta1; a.beta2 = (float)beta2; a.eps = (float)eps; a.inv_m = (float)(1.0 / (double)m_total);
+  a.stats = stats_out; a.stats_rows = stats_rows; a.stats_row = stats_row; a.epoch_end = epoch_end ? 1 : 0;
+  pop_adam_kernel<<<pop->K, 1024, 0, (cudaStream_t)stream>>>(a);
+  AUR_LAUNCH_OK("pop_adam_kernel");
   return 0;
 }

@@ -114,21 +114,33 @@ __device__ __forceinline__ void load_adv_moments(const UpdDev& a, double& s, dou
     s = a.moments[0]; ss = a.moments[1]; n = a.moments[2];
   }
 }
-__device__ __forceinline__ void adv_norm_consts(const UpdDev& a, float& mean_out, float& den_out) {
-  double s, ss, n;
-  load_adv_moments(a, s, ss, n);
+__device__ __forceinline__ void adv_norm_from_moments(double s, double ss, double n, float& mean_out, float& den_out) {
   const double mean = s / n;
   double var = (ss - s * mean) / (n - 1.0);          // unbiased (torch .std())
   if (var < 0.0) var = 0.0;
   mean_out = (float)mean;
   den_out = (float)sqrt(var) + 1e-8f;
 }
+__device__ __forceinline__ void adv_norm_consts(const UpdDev& a, float& mean_out, float& den_out) {
+  double s, ss, n;
+  load_adv_moments(a, s, ss, n);
+  adv_norm_from_moments(s, ss, n, mean_out, den_out);
+}
 #endif
 
 
 
+// population form of the tensor-core update (aur_pop_update_grad): member k = blockIdx.y reads params + k * P, idx + k * idx_stride,
+// moments + k * mom_stride and writes partials + k * part_stride; members with active[k] == 0 are skipped
+struct PopUpd {
+  const aur_pop_hparams* hp;
+  const int32_t* active;
+  long long P, idx_stride, mom_stride, part_stride;
+};
+
 // tensor-core implementation (update_tc.cu): both nets per CTA, grid = gx CTAs; same partial layout
 int launch_ppo_grad_tc(const UpdDev& d, int gx, int threads_per_sample, cudaStream_t s);
+int launch_ppo_grad_tc_pop(const UpdDev& d, const PopUpd& pop, int gx, int K, cudaStream_t s);
 size_t ppo_grad_tc_smem_bytes();
 
 }  // namespace aur

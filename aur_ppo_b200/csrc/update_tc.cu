@@ -54,6 +54,7 @@ static_assert(2 * (T2_SMEM + 1024) <= 233472, "two CTAs per SM");
 
 // small-weight block (floats): W1^T [4][64] (zero rows >= obs_dim), b1 [64], b2 [64], W3 [4][64], b3 [4]
 constexpr int S2_W1T = 0, S2_B1 = 256, S2_B2 = 320, S2_W3 = 384, S2_B3 = 640, S2_NC = 644, S2_ST = 660;   // S2_NC: Normal constants [3][4], then advantage mean / std + 1e-8; S2_ST: statistics slots [4 warps][9]
+constexpr int S2_PC = 700;                  // population form: the member's clip, clip_lo, clip_hi, ent_c, vf_c
 enum { BAR_FWD = 0, BAR_AUX = 1, BAR_WG = 2, BAR_FIN = 3 };
 constexpr int T2_TMEM_COLS = 256;           // z / dh 64 (never live together) | dW2 64 | db2 16 | [db1 dW1] 16 | h1 (fp32 copy) 64
 
@@ -95,8 +96,11 @@ __device__ __forceinline__ void mma_over_samples(uint32_t d, uint64_t a_himid, u
 }
 
 // TPS = threads per sample (2 or 4): each owns FPT = 64 / TPS hidden features of its sample.
-template <bool ACTOR, int TPS>
-__device__ __forceinline__ void tc_update_net(const UpdDev& a, unsigned char* smem_base, int cta, int ncta) {
+// POP: member blockIdx.y of a population (ppo_grad_tc_kernel<TPS, true>): its parameters, index list, moments and partial rows
+// are offset by pop's strides, its coefficients come from pop.hp and live in shared memory (S2_PC); the argument block itself is
+// never modified, so it stays in the constant bank.
+template <bool ACTOR, int TPS, bool POP>
+__device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop, unsigned char* smem_base, int cta, int ncta) {
   constexpr int THREADS = 128 * TPS, FPT = 64 / TPS, CPT = FPT / 8;
   T2Ptrs P;
   P.base = smem_base;
@@ -114,7 +118,7 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, unsigned char* sm
   if (warp == 0) tc::tmem_alloc(P.tmem_slot(), T2_TMEM_COLS);
   float* sw = P.small_w();
   {
-    const float* g = ACTOR ? a.params : a.params + gA;
+    const float* g = (POP ? a.params + blockIdx.y * pop.P : a.params) + (ACTOR ? 0 : gA);
     const float* gb1 = g + 64 * obs_dim;
     const float* gW2 = gb1 + 64;
     const float* gb2 = gW2 + 4096;
@@ -147,11 +151,24 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, unsigned char* sm
   if (tid < 256) *reinterpret_cast<unsigned short*>(P.aux(tid >> 7, 0) + aux_off(0, tid & 127)) = 0x3F80;
 
   if (ACTOR && a.continuous && tid == 0) {
-    const NormalConsts nc = normal_consts(a.params + gA + gC, A);
+    const NormalConsts nc = normal_consts((POP ? a.params + blockIdx.y * pop.P : a.params) + gA + gC, A);
 #pragma unroll
     for (int k = 0; k < POL_OUT_MAX; ++k) { sw[S2_NC + k] = nc.std[k]; sw[S2_NC + 4 + k] = nc.inv2var[k]; sw[S2_NC + 8 + k] = nc.log_scale[k]; }
   }
-  if (ACTOR && a.norm_adv && tid == 32) adv_norm_consts(a, sw[S2_NC + 12], sw[S2_NC + 13]);   // (waits for the peers' moments when data-parallel)
+  if constexpr (POP) {
+    if (ACTOR && a.norm_adv && tid == 32) {
+      const double* mom = a.moments + blockIdx.y * pop.mom_stride;
+      adv_norm_from_moments(mom[0], mom[1], mom[2], sw[S2_NC + 12], sw[S2_NC + 13]);
+    }
+    if (tid == 64) {                                   // exactly as aur_ppo_update_grad derives them from its float arguments
+      const aur_pop_hparams& h = pop.hp[blockIdx.y];
+      const float clip = (float)h.clip_coeff;
+      sw[S2_PC] = clip; sw[S2_PC + 1] = (float)(1.0 - (double)clip); sw[S2_PC + 2] = (float)(1.0 + (double)clip);
+      sw[S2_PC + 3] = (float)h.entropy_coeff; sw[S2_PC + 4] = (float)h.value_coeff;
+    }
+  } else {
+    if (ACTOR && a.norm_adv && tid == 32) adv_norm_consts(a, sw[S2_NC + 12], sw[S2_NC + 13]);   // (waits for the peers' moments when data-parallel)
+  }
   tc::fence_proxy_async();
   tc::fence_before_sync();
   __syncthreads();
@@ -198,9 +215,16 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, unsigned char* sm
   auto fetch_row = [&](long long tile) -> int {
     const long long gi = tile * T2_S + s;
     if (tile >= ntiles || gi >= a.m_local) return -1;
+    if constexpr (POP) return __ldg(a.idx + blockIdx.y * pop.idx_stride + gi);
     return a.idx ? __ldg(a.idx + gi) : (int)gi;
   };
-  const long long row_off = a.idx ? 0 : a.idx_offset;
+  const long long row_off = (POP || a.idx) ? 0 : a.idx_offset;
+  // the member's coefficients (POP: from shared memory), else the argument block's
+  auto c_clip = [&]() -> float { if constexpr (POP) return sw[S2_PC]; else return a.clip; };
+  auto c_clip_lo = [&]() -> float { if constexpr (POP) return sw[S2_PC + 1]; else return a.clip_lo; };
+  auto c_clip_hi = [&]() -> float { if constexpr (POP) return sw[S2_PC + 2]; else return a.clip_hi; };
+  auto c_ent = [&]() -> float { if constexpr (POP) return sw[S2_PC + 3]; else return a.ent_c; };
+  auto c_vf = [&]() -> float { if constexpr (POP) return sw[S2_PC + 4]; else return a.vf_c; };
   float xn[POL_IN_PAD];
   const float4* rec = ACTOR ? a.rec_actor : a.rec_critic;      // packed records: one 32-B sector per sample
   auto fetch_obs = [&](long long row) {
@@ -439,11 +463,11 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, unsigned char* sm
           }
           const float logr = newlogp - oldlp, ratio = expf(logr);
           const float advn = a.norm_adv ? (adv - adv_mean) / adv_den : adv;
-          const float l1 = -advn * ratio, l2 = -advn * fminf(fmaxf(ratio, a.clip_lo), a.clip_hi);
+          const float l1 = -advn * ratio, l2 = -advn * fminf(fmaxf(ratio, c_clip_lo()), c_clip_hi());
           const float w1 = l1 > l2 ? 1.0f : (l1 == l2 ? 0.5f : 0.0f);
-          const float inr = (ratio >= a.clip_lo && ratio <= a.clip_hi) ? 1.0f : 0.0f;
+          const float inr = (ratio >= c_clip_lo() && ratio <= c_clip_hi()) ? 1.0f : 0.0f;
           const float g_logp = -advn * (w1 + (1.0f - w1) * inr) * ratio * a.inv_m;
-          const float g_H = -a.ent_c * a.inv_m;
+          const float g_H = -c_ent() * a.inv_m;
 #pragma unroll
           for (int k = 0; k < POL_OUT_MAX; ++k) dout[k] = g_logp * dlp[k] + g_H * dH[k];
           if (a.continuous) {
@@ -451,20 +475,20 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, unsigned char* sm
             for (int k = 0; k < POL_OUT_MAX; ++k) if (k < OUT) sv[5 + k] = g_logp * g_ls[k] + g_H;
           }
           sv[0] = fmaxf(l1, l2); sv[1] = entropy; sv[2] = -logr; sv[3] = (ratio - 1.0f) - logr;
-          sv[4] = fabsf(ratio - 1.0f) > a.clip ? 1.0f : 0.0f;
+          sv[4] = fabsf(ratio - 1.0f) > c_clip() ? 1.0f : 0.0f;
         } else {
           const float R = e0, vold = e1, v = out[0];
           if (a.clip_vloss) {
             const float du = v - R, vu = du * du;
-            const float d = v - vold, vc = vold + fminf(fmaxf(d, -a.clip), a.clip);
+            const float d = v - vold, vc = vold + fminf(fmaxf(d, -c_clip()), c_clip());
             const float dc = vc - R, lc = dc * dc;
             const float w1 = vu > lc ? 1.0f : (vu == lc ? 0.5f : 0.0f);
-            const float inr = (d >= -a.clip && d <= a.clip) ? 1.0f : 0.0f;
-            dout[0] = (w1 * du + (1.0f - w1) * dc * inr) * a.vf_c * a.inv_m;
+            const float inr = (d >= -c_clip() && d <= c_clip()) ? 1.0f : 0.0f;
+            dout[0] = (w1 * du + (1.0f - w1) * dc * inr) * c_vf() * a.inv_m;
             sv[0] = 0.5f * fmaxf(vu, lc);
           } else {
             const float d = v - vold;
-            dout[0] = d * a.vf_c * a.inv_m;
+            dout[0] = d * c_vf() * a.inv_m;
             sv[0] = 0.5f * d * d;
           }
         }
@@ -600,7 +624,7 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, unsigned char* sm
   __syncthreads();
 
   // ---- epilogue: this CTA's partial sums in the net's flat parameter order
-  float* part = a.partials + ((size_t)(ACTOR ? 0 : 1) * ncta + cta) * UPD_PSTRIDE;
+  float* part = (POP ? a.partials + blockIdx.y * pop.part_stride : a.partials) + ((size_t)(ACTOR ? 0 : 1) * ncta + cta) * UPD_PSTRIDE;
   const int oB1 = 64 * obs_dim, oW2 = oB1 + 64, oB2 = oW2 + 4096, oW3 = oB2 + 64, oB3 = oW3 + OUT * 64, oLS = oB3 + OUT;
   {
     // TMEM accumulators: rows 0..63 (hi^T B) + rows 64..127 (mid^T B) = feature j; thread (row, slice) reads FPT columns
@@ -703,13 +727,18 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, unsigned char* sm
   if (warp == 0) tc::tmem_dealloc(tmem, T2_TMEM_COLS);
 }
 
-template <int TPS>
-__global__ void __launch_bounds__(128 * TPS, 2) ppo_grad_tc_kernel(UpdDev a) {
+// POP: population form (aur_pop_update_grad), grid (2 c, K): member k = blockIdx.y trains with its own parameters, index
+// list, advantage moments, coefficients and partial rows; an inactive member (target_kl) does nothing.
+template <int TPS, bool POP = false>
+__global__ void __launch_bounds__(128 * TPS, 2) ppo_grad_tc_kernel(UpdDev a, PopUpd pop) {
   extern __shared__ unsigned char smem_raw[];
   unsigned char* base = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // pointer arithmetic keeps the shared address space
   const int ncta = gridDim.x >> 1;                     // CTAs per net; blockIdx < ncta: actor, else critic
-  if ((int)blockIdx.x < ncta) tc_update_net<true, TPS>(a, base, blockIdx.x, ncta);
-  else tc_update_net<false, TPS>(a, base, blockIdx.x - ncta, ncta);
+  if constexpr (POP) {
+    if (!pop.active[blockIdx.y]) return;               // the whole CTA: a member stopped by its target_kl
+  }
+  if ((int)blockIdx.x < ncta) tc_update_net<true, TPS, POP>(a, pop, base, blockIdx.x, ncta);
+  else tc_update_net<false, TPS, POP>(a, pop, base, blockIdx.x - ncta, ncta);
 }
 
 size_t ppo_grad_tc_smem_bytes() { return T2_SMEM; }
@@ -730,9 +759,22 @@ int launch_ppo_grad_tc(const UpdDev& d, int gx, int tps, cudaStream_t s) {
     if ((rc = tc_attrs<2>()) || (rc = tc_attrs<4>())) return rc;
     attr.done();
   }
-  if (tps == 4) ppo_grad_tc_kernel<4><<<2 * gx, 512, T2_SMEM, s>>>(d);
-  else ppo_grad_tc_kernel<2><<<2 * gx, 256, T2_SMEM, s>>>(d);
+  if (tps == 4) ppo_grad_tc_kernel<4><<<2 * gx, 512, T2_SMEM, s>>>(d, PopUpd{});
+  else ppo_grad_tc_kernel<2><<<2 * gx, 256, T2_SMEM, s>>>(d, PopUpd{});
   AUR_LAUNCH_OK("ppo_grad_tc_kernel");
+  return 0;
+}
+
+// population form: gx CTAs per net and member, K members (two threads per sample)
+int launch_ppo_grad_tc_pop(const UpdDev& d, const PopUpd& pop, int gx, int K, cudaStream_t s) {
+  static DeviceOnce attr;
+  if (attr.first()) {
+    AUR_CUDA_OK(cudaFuncSetAttribute(ppo_grad_tc_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T2_SMEM));
+    AUR_CUDA_OK(cudaFuncSetAttribute(ppo_grad_tc_kernel<2, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    attr.done();
+  }
+  ppo_grad_tc_kernel<2, true><<<dim3(2 * gx, K), 256, T2_SMEM, s>>>(d, pop);
+  AUR_LAUNCH_OK("ppo_grad_tc_kernel (population)");
   return 0;
 }
 

@@ -31,11 +31,16 @@ struct VtCfg {
 static_assert(3 * (VtCfg<64>::SMEM + 1024) <= 233472, "three CTAs per SM");
 static_assert(VtCfg<128>::SMEM <= 232448, "one CTA per SM");
 
-template <int H>
+// POP: population form, grid (x, K): the rows are T segments per member of n_member rows each, segment (t, k) at rows
+// (t * K + k) * n_member ..; CTA (x, k) walks member k's tiles (at most 128 rows of one segment) with member k's critic
+// (critic + k * pop_P).  A value depends on its own row only, so it is the single run's whatever the tiling.
+template <int H, bool POP = false>
 __global__ void __launch_bounds__(VT_THREADS, VtCfg<H>::CTAS) critic_values_tc_kernel(const float* __restrict__ critic, int obs_dim,
                                                                                       const float* __restrict__ obs, long long M,
-                                                                                      float* __restrict__ out) {
+                                                                                      float* __restrict__ out, int pop_K,
+                                                                                      long long n_member, long long pop_P) {
   using Cfg = VtCfg<H>;
+  if constexpr (POP) critic += (long long)blockIdx.y * pop_P;
   constexpr int KA = Cfg::KA, FPT = Cfg::FPT;
   constexpr int VS_W1T = Cfg::S_W1T, VS_B1 = Cfg::S_B1, VS_B2 = Cfg::S_B2, VS_W3 = Cfg::S_W3, VS_B3 = Cfg::S_B3;
   extern __shared__ unsigned char smem_raw[];
@@ -79,10 +84,23 @@ __global__ void __launch_bounds__(VT_THREADS, VtCfg<H>::CTAS) critic_values_tc_k
   constexpr uint32_t ID_FWD = tc::instr_desc(tc::FMT_BF16, 128, H, 0, 0);
   const bool vec = obs_dim == 4 && (reinterpret_cast<uintptr_t>(obs) & 15) == 0;
 
-  const long long ntiles = (M + VT_S - 1) / VT_S;
+  // POP: member-local tiles, tps per segment
+  const long long tps = POP ? (n_member + VT_S - 1) / VT_S : 1;
+  const long long ntiles = POP ? (M / ((long long)pop_K * n_member)) * tps : (M + VT_S - 1) / VT_S;
+  auto tile_row = [&](long long tile, bool& ok) -> long long {
+    if constexpr (POP) {
+      const long long t = tile / tps, r = (tile - t * tps) * VT_S + s;
+      ok = tile < ntiles && r < n_member;
+      return (t * pop_K + blockIdx.y) * n_member + r;
+    } else {
+      const long long row = tile * VT_S + s;
+      ok = tile < ntiles && row < M;
+      return row;
+    }
+  };
   auto load_obs = [&](long long tile, float (&x)[POL_IN_PAD]) {
-    const long long row = tile * VT_S + s;
-    const bool ok = tile < ntiles && row < M;
+    bool ok;
+    const long long row = tile_row(tile, ok);
     if (ok && vec) {
       const float4 v = __ldg(reinterpret_cast<const float4*>(obs) + row);
       x[0] = v.x; x[1] = v.y; x[2] = v.z; x[3] = v.w;
@@ -157,8 +175,9 @@ __global__ void __launch_bounds__(VT_THREADS, VtCfg<H>::CTAS) critic_values_tc_k
     if (half == 0) {
       tc::fence_after_sync();
       const float other = tc::tmem_ld1(tm_z + lane_base + FPT);
-      const long long row = tile * VT_S + s;
-      if (row < M) out[row] = ((p0 + p1) + other) + sw[VS_B3];
+      bool ok;
+      const long long row = tile_row(tile, ok);
+      if (ok) out[row] = ((p0 + p1) + other) + sw[VS_B3];
     }
   }
   tc::fence_before_sync();
@@ -180,13 +199,33 @@ static int launch_values(const float* critic, int obs_dim, const float* obs, lon
   const long long ntiles = (M + VT_S - 1) / VT_S;
   long long grid = (long long)Cfg::CTAS * sm_count();
   if (grid > ntiles) grid = ntiles;
-  critic_values_tc_kernel<H><<<(unsigned)grid, VT_THREADS, Cfg::SMEM, s>>>(critic, obs_dim, obs, M, out);
+  critic_values_tc_kernel<H><<<(unsigned)grid, VT_THREADS, Cfg::SMEM, s>>>(critic, obs_dim, obs, M, out, 1, 0, 0);
   AUR_LAUNCH_OK("critic_values_tc_kernel");
   return 0;
 }
 int launch_critic_values_tc(const float* critic, int obs_dim, int hidden, const float* obs, long long M, float* out, cudaStream_t s) {
   if (M <= 0) return 0;
   return hidden == 128 ? launch_values<128>(critic, obs_dim, obs, M, out, s) : launch_values<64>(critic, obs_dim, obs, M, out, s);
+}
+
+// population values (aur_pop_rollout): M = segs * K * n_member rows, member k's critic at critic + k * P; about as many CTAs in
+// all as the single-run pass
+int launch_critic_values_tc_pop(const float* critic, int obs_dim, const float* obs, long long segs, int K, long long n_member,
+                                long long P, float* out, cudaStream_t s) {
+  using Cfg = VtCfg<64>;
+  static DeviceOnce attr;
+  if (attr.first()) {
+    AUR_CUDA_OK(cudaFuncSetAttribute(critic_values_tc_kernel<64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM));
+    AUR_CUDA_OK(cudaFuncSetAttribute(critic_values_tc_kernel<64, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    attr.done();
+  }
+  const long long ntiles = segs * ((n_member + VT_S - 1) / VT_S);      // per member
+  long long gx = ((long long)Cfg::CTAS * sm_count() + K - 1) / K;
+  if (gx > ntiles) gx = ntiles;
+  critic_values_tc_kernel<64, true><<<dim3((unsigned)gx, (unsigned)K), VT_THREADS, Cfg::SMEM, s>>>(
+      critic, obs_dim, obs, segs * K * n_member, out, K, n_member, P);
+  AUR_LAUNCH_OK("critic_values_tc_kernel (population)");
+  return 0;
 }
 
 }  // namespace aur

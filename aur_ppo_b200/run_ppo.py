@@ -6,12 +6,16 @@ Additions (all opt-in, none changes a reference default):
   --no_continuous_override   keep the CLI's num_envs/num_steps/... when --continuous is given
                              (the reference forces num_envs=1; BASELINE config C uses 65536)
   --no_tensorboard / --no_save
+  --population K             train K members with seeds seed, seed + 1, ... in shared launches (population.py)
+  --sweep KEY=V1,V2,...      repeatable: a population over the cartesian product of the listed per-member values
+                             (learning_rate, entropy_coeff, clip_coeff, value_coeff, max_grad_norm, target_kl) and the seeds
 """
 from __future__ import annotations
 
 import argparse
+import itertools
 import sys
-from typing import Dict, List, Optional
+from typing import Dict, List, Optional, Sequence
 
 
 def strtobool(val: str) -> int:
@@ -59,7 +63,45 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument('--no_continuous_override', action='store_true', help='keep CLI sizes when --continuous is set')
     p.add_argument('--no_tensorboard', action='store_true')
     p.add_argument('--no_save', action='store_true')
+    p.add_argument('--population', type=int, default=0, help='train this many members (seeds seed, seed+1, ...) at once')
+    p.add_argument('--sweep', action='append', default=[], metavar='KEY=V1,V2,...',
+                   help='per-member values of KEY (repeatable; cartesian product with the population seeds)')
     return p
+
+
+SWEEP_KEYS = ("learning_rate", "entropy_coeff", "clip_coeff", "value_coeff", "max_grad_norm", "target_kl")
+
+
+def expand_members(seed: float, population: int, sweeps: Sequence[str]) -> List[Dict]:
+    """--population / --sweep -> the member override dicts of a population: for every combination of the swept values (in
+    the order the flags are given), `population` members (at least one) with seeds seed, seed + 1, ...  Empty when neither flag
+    is used (a single run)."""
+    if population < 0:
+        raise ValueError("--population must be >= 0")
+    if not population and not sweeps:
+        return []
+    axes = []
+    for spec in sweeps:
+        key, sep, vals = spec.partition("=")
+        key = key.strip()
+        if not sep or key not in SWEEP_KEYS:
+            raise ValueError(f"--sweep {spec!r}: expected KEY=V1,V2,... with KEY one of {', '.join(SWEEP_KEYS)}")
+        if key in (k for k, _ in axes):
+            raise ValueError(f"--sweep {key} given twice")
+        parsed = []
+        for v in vals.split(","):
+            v = v.strip()
+            if not v:
+                raise ValueError(f"--sweep {spec!r}: empty value")
+            parsed.append(None if key == "target_kl" and v.lower() == "none" else float(v))
+        axes.append((key, parsed))
+    members = []
+    for combo in itertools.product(*[vals for _, vals in axes]):
+        for i in range(max(population, 1)):
+            m = {"seed": seed + i}
+            m.update({key: v for (key, _), v in zip(axes, combo)})
+            members.append(m)
+    return members
 
 
 def params_from_args(args: argparse.Namespace) -> Dict:
@@ -89,8 +131,16 @@ def params_from_args(args: argparse.Namespace) -> Dict:
 
 
 def main(argv: Optional[List[str]] = None):
-    args = build_parser().parse_args(argv)
+    parser = build_parser()
+    args = parser.parse_args(argv)
     params = params_from_args(args)
+    try:
+        members = expand_members(args.seed, args.population, args.sweep)
+    except ValueError as e:
+        parser.error(str(e))
+    if members:
+        from .population import ppo_population
+        return ppo_population(params, members).train()
     from .ppo import ppo
     to_run = ppo(params)
     return to_run.train()

@@ -339,6 +339,103 @@ int aur_ppo_update_apply_dp(const aur_policy_desc* desc, float* params, float* g
                             double max_grad_norm, int64_t m_total, double entropy_coeff, double value_coeff,
                             float* stats_out, const aur_dp_ctx* dp, uint32_t seq, void* stream);
 
+/* ---------------------------------------------------------- populations ----
+ * K independent PPO runs ("members") trained in shared launches on one GPU: the seed / hyper-parameter sweeps of the
+ * reference (src/grid_search.sh, src/robot.sh; `--trials`, src/run_ppo.py:41) as one set of kernels instead of K processes.
+ * Members share the policy shape, the env and every size (num_envs = n_member, num_steps, minibatches, epochs); each has its
+ * own parameters, Adam moments, Philox / shuffle key and the hyper-parameters of aur_pop_hparams.  Member k computes exactly
+ * (bit for bit) what the single-run entry points compute for a run of n_member envs with philox_seed = shuffle_seed =
+ * seeds[k] started from the same parameters: the same kernels run with per-member operands, the update splits each member's
+ * minibatch over min(#SM, tiles) CTAs per net exactly as a single run does, and every fp64 reduction keeps its single-run order.
+ *
+ * Scope: hidden 64, 2 layers, obs_dim <= 4, act_dim <= 4 (act_dim <= 2 if continuous), CartPole-v1, Pendulum-v1 (with or
+ * without the wrapper stack) and MountainCar-v0, one GPU.  Anything else returns AUR_ERR_UNSUPPORTED; there is no fallback.
+ * Populations always run the tensor-core kernels: aur_rollout_set_impl / aur_ppo_update_set_impl do not apply to them.
+ *
+ * Layout: the rollout buffers are the single-run buffers of N = K * n_member envs ([T][K * n_member], member k owns columns
+ * k * n_member .. (k+1) * n_member - 1), so aur_gae_f32 and aur_ppo_pack_records run on them unchanged, as one launch each.
+ * Per-member device arrays are stacked along a leading K axis (parameters [K][P], Adam moments [K][P], gradients
+ * [K][P + 16], ...).  Last-CTA tickets are not used: the workspace needs no initialisation. */
+typedef struct {
+  int32_t K;               /* members, >= 1 */
+  int32_t _pad;
+  int64_t n_member;        /* envs per member, >= 1 (any value: a CTA never straddles two members) */
+  const uint64_t* seeds;   /* [K] device: member k's Philox sampling key and shuffle key */
+} aur_pop_desc;
+
+/* One member's hyper-parameters (src/run_ppo.py:21-31 flags), a device table [K] written once. */
+typedef struct {
+  double learning_rate;    /* before the anneal factor: the step uses (float)((learning_rate * frac) / bias_correction1) */
+  double entropy_coeff;
+  double clip_coeff;
+  double value_coeff;
+  double max_grad_norm;
+  double target_kl;        /* +inf: no early stop (the reference's None) */
+} aur_pop_hparams;
+
+/* Replaces the rollout loop (src/ppo.py:201-205) of every member in one launch of the fused tensor-core rollout kernel, grid
+ * (ceil(n_member / 128), K), followed by the batched critic pass.  `args` is as for aur_rollout with N = K * n_member and:
+ *   params       [K][P]: member k's flat parameter buffer at params + k * P
+ *   seed         ignored: member k samples from Philox(key = pop->seeds[k], counter = (env_id0 + n, step0 + t)), n the
+ *                member-local env index - the counters of a single run of n_member envs
+ *   log          first_finished [K][T] (caller-initialised to all ones), totals [K][3] (or NULL); keys hold the member-local
+ *                env index.  entries / count must be NULL.
+ * Env state, next_obs / next_done / next_value and the buffers span all K * n_member columns.
+ * AUR_ERR_UNSUPPORTED outside the population scope, AUR_ERR_ARG for bad pointers / sizes. */
+int aur_pop_rollout(const aur_pop_desc* pop, const aur_rollout_args* args, void* stream);
+
+/* `np.random.shuffle(b_inds)` (ppo.py:214-215) of `epochs` consecutive epochs for every member in one launch: member k's
+ * epoch e is the permutation aur_shuffle_indices(T * n_member, pop->seeds[k], stream_id0 + e) of its local batch, each local
+ * index j written as the GLOBAL row (j / n_member) * (K * n_member) + k * n_member + j % n_member of the population batch.
+ * out: [K][epochs][T * n_member] int32.  T * n_member < 2^31, K * T * n_member < 2^31. */
+int aur_pop_shuffle_indices(const aur_pop_desc* pop, int32_t T, int32_t epochs, uint64_t stream_id0, int32_t* out, void* stream);
+
+/* aur_ppo_adv_moments_multi for every member (ppo.py:239 `mb_advantages.mean() / .std()` of the whole update loop): idx
+ * [K][n_mb][m] global rows, moments_out [K][n_mb][3].  Each member is split over the CTAs a single run would use, and the
+ * fp64 partials are combined in the single-run order.  Two launches, whatever K. */
+int aur_pop_adv_moments_multi(const aur_pop_desc* pop, int32_t n_mb, int64_t m, const int32_t* idx, const float* advantages,
+                              double* moments_out, float* workspace, void* stream);
+
+typedef struct {
+  aur_policy_desc policy;
+  int32_t norm_adv;          /* ppo.py:238 */
+  int32_t clip_vloss;        /* ppo.py:250 */
+  int32_t mb_index;          /* minibatch j of the iteration: index list j and moments entry j of every member */
+  int32_t n_mb;              /* minibatches per iteration (entries per member of idx / adv_moments) */
+  int64_t m;                 /* samples per minibatch and member (means divide by this) */
+  const int32_t* idx;        /* [K][n_mb][m] global rows (aur_pop_shuffle_indices) */
+  const float* rec_actor;    /* [K * T * n_member][8] records of aur_ppo_pack_records over the population batch (required) */
+  const float* rec_critic;
+  const float* params;       /* [K][P] */
+  const aur_pop_hparams* hparams;   /* [K] device */
+  const double* adv_moments; /* [K][n_mb][3] (aur_pop_adv_moments_multi); NULL iff !norm_adv */
+  const int32_t* active;     /* [K] device: members with 0 are skipped (target_kl, aur_pop_update_apply) */
+  float* workspace;          /* >= aur_pop_update_workspace_bytes(); contents need not be initialised */
+  float* grads_out;          /* [K][P + 16]: member k's [gradient sums | statistic sums] */
+} aur_pop_update_args;
+
+/* Workspace of aur_pop_adv_moments_multi / aur_pop_update_grad for K members, n_mb minibatches of m samples. */
+int64_t aur_pop_update_workspace_bytes(const aur_pop_desc* pop, const aur_policy_desc* desc, int32_t n_mb, int64_t m);
+
+/* aur_ppo_update_grad for one minibatch of every active member: gather + forward + loss + backward on the tensor cores, grid
+ * (2 c, K) with c = min(#SM, ceil(m / 128)) CTAs per net (tile i on CTA i mod c, as a single run), then one fixed-order fp64
+ * reduction per member that keeps the single-run quarter boundaries.  Two launches, whatever K. */
+int aur_pop_update_grad(const aur_pop_desc* pop, const aur_pop_update_args* args, void* stream);
+
+/* clip_grad_norm_ + Adam (ppo.py:266-269) for every active member, one CTA each.  Member k steps with lr = (float)(
+ * (hparams[k].learning_rate * frac) / bc[s][0]), bc[s][1] = 1 - beta2^s under the sqrt, s = steps[k] + 1 its 1-based Adam step
+ * (bc [bc_len][2] fp64, a host-computed table of 1 - beta1^s, 1 - beta2^s: the values aur_ppo_update_apply derives with host
+ * pow), then steps[k] = s.  The caller keeps bc_len > the largest step any member can reach (at most the number of apply calls
+ * made so far); a member whose next step has no table entry is NOT stepped (its parameters, moments and step count stay as
+ * they are), so a short table shows as a step count that stops advancing.  stats_out [K][stats_rows][16]: row stats_row of member k receives its minibatch means.  epoch_end
+ * != 0 (the last minibatch of an epoch): a member whose approx_kl exceeds hparams[k].target_kl is cleared in `active`
+ * (ppo.py:271-273 `break`), so its later grad / apply work of the iteration is skipped and its step count stops.
+ * params / adam_m / adam_v [K][P], grads [K][P + 16], steps [K] int64 device. */
+int aur_pop_update_apply(const aur_pop_desc* pop, const aur_policy_desc* desc, const aur_pop_hparams* hparams, float* params,
+                         const float* grads, float* adam_m, float* adam_v, int64_t* steps, int32_t* active, const double* bc,
+                         int64_t bc_len, double frac, double beta1, double beta2, double eps, int64_t m_total,
+                         float* stats_out, int32_t stats_rows, int32_t stats_row, int32_t epoch_end, void* stream);
+
 /* ------------------------------------------------ squashed Gaussian head ----
  * PPOGaussianPolicyBase.sample (src/nets/nets.py:90-105): y = tanh(action), log_prob = sum_k Normal(mean,
  * exp(log_std)).log_prob(action) - log(1 - y^2 + 1e-6) ([B], the reference keeps dim 1), tanh(mean), and the
