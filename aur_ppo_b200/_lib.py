@@ -71,6 +71,13 @@ class PopUpdateArgs(ctypes.Structure):
                 ("grads_out", c_void_p)]
 
 
+class PopPbtArgs(ctypes.Structure):
+    _fields_ = [("fitness", c_void_p), ("q", c_double), ("down", c_double), ("up", c_double), ("mask", ctypes.c_uint32),
+                ("_pad", ctypes.c_uint32), ("seed", c_uint64), ("round", c_uint64), ("params", c_void_p), ("adam_m", c_void_p),
+                ("adam_v", c_void_p), ("steps", c_void_p), ("hparams", c_void_p), ("norm", c_void_p), ("norm_ld", c_int64),
+                ("rank_out", c_void_p), ("donor_out", c_void_p), ("order", c_void_p)]
+
+
 DP_MAX_RANKS = 16
 DP_HANDLE_BYTES = 64
 
@@ -274,6 +281,10 @@ def lib() -> ctypes.CDLL:
     L.aur_pop_update_apply.argtypes = [ctypes.POINTER(PopDesc), ctypes.POINTER(PolicyDesc), c_void_p, c_void_p, c_void_p, c_void_p,
                                        c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_double, c_double, c_double, c_double,
                                        c_int64, c_void_p, c_int32, c_int32, c_int32, c_void_p]
+    L.aur_pop_episode_fitness.restype = c_int
+    L.aur_pop_episode_fitness.argtypes = [ctypes.POINTER(PopDesc), c_void_p, c_void_p, c_void_p, c_void_p]
+    L.aur_pop_pbt_step.restype = c_int
+    L.aur_pop_pbt_step.argtypes = [ctypes.POINTER(PopDesc), ctypes.POINTER(PolicyDesc), ctypes.POINTER(PopPbtArgs), c_void_p]
     L.aur_sincos_f64.restype = c_int
     L.aur_sincos_f64.argtypes = [c_int64, c_void_p, c_void_p, c_void_p, c_void_p]
     _lib = L

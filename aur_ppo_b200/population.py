@@ -10,12 +10,19 @@ value coefficients, max_grad_norm and target_kl; everything else is shared.  Mem
   per iteration            one aur_pop_rollout, one aur_gae_f32, one aur_ppo_pack_records, one aur_pop_shuffle_indices,
                            one aur_pop_adv_moments_multi (all members, all minibatches)
   per minibatch            one aur_pop_update_grad (all members), one aur_pop_update_apply (all members)
+  per PBT round (opt-in)   one aur_pop_episode_fitness, one aur_pop_pbt_step (two launches), between iterations
+
+Population-based training (`pbt=dict(interval=...)`): every `interval` iterations the bottom `fraction` of the members (by the
+mean return of the episodes they finished since the last round) copy the weights, Adam state and wrapper statistics of
+members drawn from the top `fraction`, then multiply the copied hyper-parameters named in `keys` by one of `factors`
+(include/aur_ppo.h, "population-based training").  With `pbt=None` nothing changes.
 
 Layout: the rollout buffers are those of a single run of K * n_member envs; member k owns columns k * n_member ...
 """
 from __future__ import annotations
 
 import ctypes
+import json
 import math
 import time
 from typing import Dict, List, Optional, Sequence
@@ -27,10 +34,12 @@ from . import _lib, compat, kernels, parallel
 from .envs import DeviceVecEnv, pcg64_seed_states
 from .models.actor_critic import actor_critic
 from .ppo import _SPACES, torch_buffer
+from .run_ppo import SWEEP_KEYS
 
 # the keys a member may set; every other key of `params` is shared by the whole population
 MEMBER_KEYS = ("seed", "learning_rate", "entropy_coeff", "clip_coeff", "value_coeff", "max_grad_norm", "target_kl")
 POP_ENVS = ("CartPole-v1", "Pendulum-v1", "MountainCar-v0")
+PBT_DEFAULTS = dict(fraction=0.25, keys=("learning_rate", "entropy_coeff"), factors=(0.8, 1.2))
 ADAM_BETAS, ADAM_EPS = (0.9, 0.999), 1e-5
 
 
@@ -57,6 +66,38 @@ def check_members(params: Dict, members: Sequence[Dict]) -> List[Dict]:
     return out
 
 
+def check_pbt(pbt: Optional[Dict], K: int) -> Optional[Dict]:
+    """Validate a PBT config (AurError) -> dict(interval, fraction, keys, factors, mask) with the defaults filled in."""
+    if pbt is None:
+        return None
+    if not isinstance(pbt, dict):
+        raise _lib.AurError(f"pbt: expected a dict, got {type(pbt).__name__}")
+    unknown = set(pbt) - {"interval", *PBT_DEFAULTS}
+    if unknown:
+        raise _lib.AurError(f"pbt: unknown settings {sorted(unknown)} (interval, fraction, keys, factors)")
+    cfg = dict(PBT_DEFAULTS, **pbt)
+    if K < 2:
+        raise _lib.AurError(f"pbt needs a population of at least two members (got {K})")
+    interval = cfg.get("interval")
+    if isinstance(interval, bool) or not isinstance(interval, int) or interval < 1:
+        raise _lib.AurError(f"pbt interval must be an integer >= 1 (got {interval!r})")
+    q = cfg["fraction"]
+    if isinstance(q, bool) or not isinstance(q, (int, float)) or not 0.0 < q <= 0.5:
+        raise _lib.AurError(f"pbt fraction must be in (0, 0.5] (got {q!r})")
+    keys = (cfg["keys"],) if isinstance(cfg["keys"], str) else tuple(cfg["keys"])
+    bad = [k for k in keys if k not in SWEEP_KEYS]
+    if bad:
+        raise _lib.AurError(f"pbt keys {bad} are not hyper-parameters a member has (one of {', '.join(SWEEP_KEYS)})")
+    try:
+        down, up = (float(v) for v in cfg["factors"])
+    except (TypeError, ValueError):
+        raise _lib.AurError(f"pbt factors must be two numbers (got {cfg['factors']!r})")
+    if not all(math.isfinite(v) and v > 0 for v in (down, up)):
+        raise _lib.AurError(f"pbt factors must be finite and > 0 (got {down}, {up})")
+    return dict(interval=interval, fraction=float(q), keys=keys, factors=(down, up),
+                mask=sum(1 << SWEEP_KEYS.index(k) for k in set(keys)))
+
+
 def _bind_flat(policy: actor_critic, row: torch.Tensor) -> None:
     """Make every parameter of `policy` a view of `row` (the flat_parameters() order) after copying its values there."""
     flat = policy.flat_parameters()
@@ -68,11 +109,12 @@ def _bind_flat(policy: actor_critic, row: torch.Tensor) -> None:
 
 
 class ppo_population:
-    def __init__(self, params: Dict, members: Sequence[Dict]):
+    def __init__(self, params: Dict, members: Sequence[Dict], pbt: Optional[Dict] = None):
         self.params_dict = params
         self.members = check_members(params, members)
         self.member_params = [member_params(params, m) for m in self.members]
         self.K = K = len(self.members)
+        self.pbt = check_pbt(pbt, K)
         for key in ("gym_id", "num_envs", "num_steps", "num_minibatches", "num_update_epochs", "gamma", "gae_lambda", "gae",
                     "norm_adv", "clip_vloss", "anneal_lr", "total_timesteps", "hidden_dim", "num_layers", "continuous", "exp_name"):
             setattr(self, key, params[key])
@@ -167,6 +209,15 @@ class ppo_population:
         self.total_returns: List[List[float]] = [[] for _ in range(K)]
         self.total_episode_lengths: List[List[int]] = [[] for _ in range(K)]
         self.x_indices: List[List[int]] = [[] for _ in range(K)]
+        # PBT: the fitness snapshot of the episode totals, the round's outputs and the history of rounds
+        self.pbt_round = 0
+        self.lineage: List[Dict] = []
+        if self.pbt is not None:
+            self.pbt_snapshot = torch.zeros(K, 3, dtype=torch.float64, device=dev)
+            self.pbt_fitness = torch.empty(K, dtype=torch.float64, device=dev)
+            self.pbt_rank = torch.empty(K, dtype=torch.int32, device=dev)
+            self.pbt_donor = torch.empty(K, dtype=torch.int32, device=dev)
+            self.pbt_order = torch.empty(K + 1, dtype=torch.int32, device=dev)
 
     def _ensure_bias_corr(self, max_step: int) -> None:
         """Adam bias corrections 1 - beta^s for s = 0 .. max_step (aur_pop_update_apply reads entry steps[k] + 1, which must exist),
@@ -275,6 +326,52 @@ class ppo_population:
         rec(3)
         return dict(stats=self._stats_rows, b_values=flat[5], b_returns=flat[4])
 
+    def pbt_step(self, fitness: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+        """One PBT round between iterations (three launches): fitness (aur_pop_episode_fitness, the mean return of each member's
+        episodes since the previous round) unless a [K] fp64 device tensor is given, then rank + exploit / explore
+        (aur_pop_pbt_step) keyed by the population's seed and the round number.  Returns device tensors donor [K] int32 (-1:
+        kept its own state), fitness [K] fp64 and rank [K] int32."""
+        if self.pbt is None:
+            raise _lib.AurError("pbt_step: this population was built without a pbt config")
+        cfg = self.pbt
+        L = _lib.lib()
+        st = kernels._stream()
+        with torch.cuda.device(self.device):
+            if fitness is None:
+                _lib.check(L.aur_pop_episode_fitness(ctypes.byref(self.pop), self.totals.data_ptr(), self.pbt_snapshot.data_ptr(),
+                                                     self.pbt_fitness.data_ptr(), st), "aur_pop_episode_fitness")
+                fitness = self.pbt_fitness
+            elif fitness.dtype != torch.float64 or fitness.shape != (self.K,) or fitness.device != self.device:
+                raise _lib.AurError(f"pbt_step: fitness must be a [{self.K}] float64 tensor on {self.device}")
+            fitness = fitness.contiguous()
+            self.pbt_round += 1
+            a = _lib.PopPbtArgs()
+            a.fitness = fitness.data_ptr()
+            a.q, (a.down, a.up), a.mask = cfg["fraction"], cfg["factors"], cfg["mask"]
+            a.seed, a.round = int(self.params_dict["seed"]) & 0xFFFFFFFFFFFFFFFF, self.pbt_round
+            a.params, a.adam_m, a.adam_v = self.params.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr()
+            a.steps, a.hparams = self.steps.data_ptr(), self.hparams.data_ptr()
+            a.norm = self.envs.norm.data_ptr() if self.envs.norm is not None else None
+            a.norm_ld = self.K * self.n_member
+            a.rank_out, a.donor_out, a.order = self.pbt_rank.data_ptr(), self.pbt_donor.data_ptr(), self.pbt_order.data_ptr()
+            _lib.check(L.aur_pop_pbt_step(ctypes.byref(self.pop), ctypes.byref(self.desc), ctypes.byref(a), st), "aur_pop_pbt_step")
+        return dict(donor=self.pbt_donor, fitness=fitness, rank=self.pbt_rank)
+
+    def _record_round(self, iteration: int, out: Dict[str, torch.Tensor]) -> Dict:
+        """Read a round's donors, fitness and hyper-parameter table back once; update member_params and the lineage."""
+        donor = out["donor"].cpu().numpy()
+        fitness = out["fitness"].cpu().numpy()
+        hp = self.hparams.cpu().numpy()
+        for k, mp in enumerate(self.member_params):
+            mp.update({key: float(hp[k, j]) for j, key in enumerate(SWEEP_KEYS)})
+            if math.isinf(mp["target_kl"]):
+                mp["target_kl"] = None
+        self.any_target_kl = any(mp["target_kl"] is not None for mp in self.member_params)
+        entry = dict(iteration=int(iteration), fitness=[None if math.isnan(f) else float(f) for f in fitness],
+                     donor=[int(d) for d in donor], hparams=[{key: mp[key] for key in SWEEP_KEYS} for mp in self.member_params])
+        self.lineage.append(entry)
+        return entry
+
     # --------------------------------------------------------------------------- train
     def member_slice(self, t: torch.Tensor, k: int) -> torch.Tensor:
         """Member k's [T, n_member, ...] part of a [T, K * n_member, ...] population buffer."""
@@ -333,12 +430,22 @@ class ppo_population:
                     w.add_scalar("losses/clipfrac", host_stats[k, :r, 5].mean(), global_step)
                     w.add_scalar("losses/explained_variance", explained_var, global_step)
                     w.add_scalar("charts/SPS", int(global_step / (time.time() - start_time)), global_step)
+            if self.pbt is not None and update % self.pbt["interval"] == 0 and update < self.num_updates:
+                entry = self._record_round(update, self.pbt_step())
+                for k, w in enumerate(writers):
+                    if w is not None:
+                        f = entry["fitness"][k]
+                        w.add_scalar("pbt/fitness", float("nan") if f is None else f, global_step)
+                        w.add_scalar("pbt/donor", entry["donor"][k], global_step)
         for w in writers:
             if w is not None:
                 w.close()
         if self.params_dict.get("save", True):
             for k in range(K):
                 compat.save_policy(self.standalone_policy(k), f"actor_critic_{self.num_layers}_m{k}.pt")
+            if self.pbt is not None:
+                with open("pbt_lineage.json", "w") as f:
+                    json.dump(self.lineage, f, indent=1)
         return [(self.total_returns[k], self.total_episode_lengths[k], self.x_indices[k]) for k in range(K)]
 
     def standalone_policy(self, k: int) -> actor_critic:

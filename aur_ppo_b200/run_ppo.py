@@ -9,6 +9,12 @@ Additions (all opt-in, none changes a reference default):
   --population K             train K members with seeds seed, seed + 1, ... in shared launches (population.py)
   --sweep KEY=V1,V2,...      repeatable: a population over the cartesian product of the listed per-member values
                              (learning_rate, entropy_coeff, clip_coeff, value_coeff, max_grad_norm, target_kl) and the seeds
+  --pbt_interval N           population-based training: every N iterations the worst members copy the weights and optimizer
+                             state of the best ones and perturb the copied hyper-parameters (0 = off, the default; needs a
+                             population of at least two members; writes pbt_lineage.json next to the checkpoints)
+  --pbt_fraction Q           the share of members that copy, and that are copied from, each round (0 < Q <= 0.5; 0.25)
+  --pbt_keys K1,K2           the hyper-parameters a copy perturbs by x0.8 or x1.2 (per-member keys above;
+                             learning_rate,entropy_coeff)
 """
 from __future__ import annotations
 
@@ -66,6 +72,9 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument('--population', type=int, default=0, help='train this many members (seeds seed, seed+1, ...) at once')
     p.add_argument('--sweep', action='append', default=[], metavar='KEY=V1,V2,...',
                    help='per-member values of KEY (repeatable; cartesian product with the population seeds)')
+    p.add_argument('--pbt_interval', type=int, default=0, help='population-based training every N iterations (0 = off)')
+    p.add_argument('--pbt_fraction', type=float, default=0.25, help='share of members replaced per PBT round, in (0, 0.5]')
+    p.add_argument('--pbt_keys', type=str, default='learning_rate,entropy_coeff', help='hyper-parameters a PBT copy perturbs')
     return p
 
 
@@ -104,6 +113,23 @@ def expand_members(seed: float, population: int, sweeps: Sequence[str]) -> List[
     return members
 
 
+def pbt_from_args(args: argparse.Namespace, n_members: int) -> Optional[Dict]:
+    """--pbt_* -> the `pbt` dict of ppo_population, or None when --pbt_interval is 0 (ValueError on a bad request)."""
+    if args.pbt_interval < 0:
+        raise ValueError("--pbt_interval must be >= 0")
+    if not args.pbt_interval:
+        return None
+    if n_members < 2:
+        raise ValueError("--pbt_interval needs --population / --sweep giving at least two members")
+    if not 0.0 < args.pbt_fraction <= 0.5:
+        raise ValueError(f"--pbt_fraction must be in (0, 0.5] (got {args.pbt_fraction})")
+    keys = tuple(k.strip() for k in args.pbt_keys.split(",") if k.strip())
+    bad = [k for k in keys if k not in SWEEP_KEYS]
+    if bad:
+        raise ValueError(f"--pbt_keys {','.join(bad)}: expected keys among {', '.join(SWEEP_KEYS)}")
+    return dict(interval=args.pbt_interval, fraction=args.pbt_fraction, keys=keys)
+
+
 def params_from_args(args: argparse.Namespace) -> Dict:
     if args.continuous and not getattr(args, "no_continuous_override", False):
         args.learning_rate = 3e-4            # run_ppo.py:44-51
@@ -136,11 +162,12 @@ def main(argv: Optional[List[str]] = None):
     params = params_from_args(args)
     try:
         members = expand_members(args.seed, args.population, args.sweep)
+        pbt = pbt_from_args(args, len(members))
     except ValueError as e:
         parser.error(str(e))
     if members:
         from .population import ppo_population
-        return ppo_population(params, members).train()
+        return ppo_population(params, members, pbt=pbt).train()
     from .ppo import ppo
     to_run = ppo(params)
     return to_run.train()

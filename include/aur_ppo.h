@@ -436,6 +436,65 @@ int aur_pop_update_apply(const aur_pop_desc* pop, const aur_policy_desc* desc, c
                          int64_t bc_len, double frac, double beta1, double beta2, double eps, int64_t m_total,
                          float* stats_out, int32_t stats_rows, int32_t stats_row, int32_t epoch_end, void* stream);
 
+/* ------------------------------------------------ population-based training ----
+ * PBT (Jaderberg et al., 2017) between two population iterations, never inside one: the worst members copy the weights and
+ * optimizer state of the best ones ("exploit"), then perturb the copied hyper-parameters ("explore").  Everything stays in
+ * the population's stacked [K][...] device arrays; a round is three launches whatever K is (aur_pop_episode_fitness: one,
+ * aur_pop_pbt_step: two).
+ *
+ * Decision rule of a round, from fitness[K] (fp64), a fraction q, factors down / up, a perturb mask over the six fields of
+ * aur_pop_hparams (bit j = field j in declaration order), a 64-bit seed and the round number r (1, 2, ...):
+ *   1. member k is ranked when fitness[k] is not NaN (+-inf are ranked); n_valid = the number of ranked members.
+ *   2. order = the ranked members sorted by fitness, highest first; ties (-0.0 == +0.0 included) go to the lower member
+ *      index.  rank[k] = k's position in order, -1 when k is not ranked.
+ *   3. n_sel = floor(q * n_valid) in fp64, 0 < q <= 0.5.  n_sel == 0: the round changes nothing.
+ *   4. k is a recipient when rank[k] >= n_valid - n_sel (the bottom n_sel); donors are the top n_sel.  q <= 0.5, so no
+ *      member is both, and every copy runs in one pass.
+ *   5. recipient k draws w = philox4x32_10(counter (k, (uint32) r, (uint32)(r >> 32), AUR_PBT_PHILOX_C3),
+ *      key ((uint32) seed, (uint32)(seed >> 32))); donor = order[((uint64) w0 * n_sel) >> 32].  Every field j of the donor's
+ *      aur_pop_hparams is copied; a field whose mask bit is set is then multiplied in fp64 by ((w1 >> j) & 1) ? up : down
+ *      (target_kl = +inf stays +inf).
+ *   6. the recipient receives the donor's parameter row, adam_m row, adam_v row and Adam step count (the bias correction
+ *      continues as the donor's) and, with the continuous wrapper stack, rows 0 .. 2D + 3 of the donor's env columns of
+ *      `norm` (observation mean / var / count, return-rms mean / var / count: donor column d * n_member + j -> recipient
+ *      column k * n_member + j) -- what the copied policy and critic were trained against.  It keeps its own seed (Philox
+ *      and shuffle key), env physics, PCG state, TimeLimit counters, episode accumulators and row 2D + 4 of `norm` (the
+ *      discounted-return accumulator of its own running episodes).
+ * oracle/pbt_ref.py restates steps 1-6. */
+#define AUR_PBT_PHILOX_C3 0x50B7D0E5u   /* fixed fourth counter word of the recipient's draw */
+
+/* The default fitness: fitness_out[k] = mean return of the episodes member k finished since the last call, from the delta
+ * of the rollout's cumulative totals [K][3] (count, return sum, length sum; aur_pop_rollout's log.totals) against snapshot
+ * [K][3] (zeros before the first call); NaN when no episode finished.  snapshot is then set to totals.  One launch.
+ * totals is accumulated with fp64 atomicAdd, so for non-integer returns (Pendulum) the last bits of a sum can depend on
+ * arrival order; integer-return envs (CartPole, MountainCar) are exact. */
+int aur_pop_episode_fitness(const aur_pop_desc* pop, const double* totals, double* snapshot, double* fitness_out, void* stream);
+
+typedef struct {
+  const double* fitness;     /* [K] device, any metric (higher is better; NaN = not ranked) */
+  double q;                  /* fraction, 0 < q <= 0.5 */
+  double down, up;           /* perturb factors, finite and > 0 */
+  uint32_t mask;             /* fields of aur_pop_hparams to perturb, bits 0..5 */
+  uint32_t _pad;
+  uint64_t seed;             /* Philox key of the draws */
+  uint64_t round;            /* r = 1, 2, ...: Philox counter of the draws */
+  float* params;             /* [K][P] */
+  float* adam_m;             /* [K][P] */
+  float* adam_v;             /* [K][P] */
+  int64_t* steps;            /* [K] Adam step counts */
+  aur_pop_hparams* hparams;  /* [K] */
+  double* norm;              /* aur_env_state.norm [2 D + 5][norm_ld] of the K * n_member envs, or NULL without wrappers */
+  int64_t norm_ld;           /* >= K * n_member when norm is given */
+  int32_t* rank_out;         /* [K]: rank[k], -1 when not ranked */
+  int32_t* donor_out;        /* [K]: the donor of recipient k, -1 for every other member */
+  int32_t* order;            /* [K + 1] scratch: order[0 .. n_valid - 1], then order[K] = n_valid */
+} aur_pop_pbt_args;
+
+/* One PBT round (rank, then exploit / explore) on the population's device arrays, two launches.  AUR_ERR_ARG without touching
+ * the device for q outside (0, 0.5], a factor <= 0 or not finite, mask bits above 5, null required pointers or a short
+ * norm_ld; AUR_ERR_UNSUPPORTED for a policy outside the population scope. */
+int aur_pop_pbt_step(const aur_pop_desc* pop, const aur_policy_desc* desc, const aur_pop_pbt_args* args, void* stream);
+
 /* ------------------------------------------------ squashed Gaussian head ----
  * PPOGaussianPolicyBase.sample (src/nets/nets.py:90-105): y = tanh(action), log_prob = sum_k Normal(mean,
  * exp(log_std)).log_prob(action) - log(1 - y^2 + 1e-6) ([B], the reference keeps dim 1), tanh(mean), and the
