@@ -79,9 +79,9 @@ __global__ void __launch_bounds__(RT_S, RtCfg<H>::CTAS) rollout_tc_kernel(Rollou
 #pragma unroll 1
     for (int e = tid; e < H * (H / 8); e += RT_S) {         // W2 row j, 8-feature chunk ch -> K atom ch / 8
       const int j = e % H, ch = e / H;
-      float v[8];
+      float2 v[4];
 #pragma unroll
-      for (int q = 0; q < 8; ++q) v[q] = gW2[j * H + 8 * ch + q];
+      for (int q = 0; q < 4; ++q) v[q] = make_float2(gW2[j * H + 8 * ch + 2 * q], gW2[j * H + 8 * ch + 2 * q + 1]);
       store_split_chunk(w2t[0] + (ch >> 3) * Cfg::WTILE, w2t[1] + (ch >> 3) * Cfg::WTILE, j, ch & 7, v);
     }
   }
@@ -133,7 +133,7 @@ __global__ void __launch_bounds__(RT_S, RtCfg<H>::CTAS) rollout_tc_kernel(Rollou
     if constexpr (!EXT) {
 #pragma unroll
     for (int c = 0; c < H / 8; ++c) {
-      float hv[8];
+      float2 hv[4];
 #pragma unroll
       for (int g = 0; g < 2; ++g) {
         const int f = 8 * c + 4 * g;
@@ -146,8 +146,8 @@ __global__ void __launch_bounds__(RT_S, RtCfg<H>::CTAS) rollout_tc_kernel(Rollou
           a01 = __ffma2_rn(make_float2(w.x, w.y), xx, a01);
           a23 = __ffma2_rn(make_float2(w.z, w.w), xx, a23);
         }
-        hv[4 * g] = tanh_prescaled(a01.x); hv[4 * g + 1] = tanh_prescaled(a01.y);
-        hv[4 * g + 2] = tanh_prescaled(a23.x); hv[4 * g + 3] = tanh_prescaled(a23.y);
+        hv[2 * g] = tanh_prescaled2(a01);
+        hv[2 * g + 1] = tanh_prescaled2(a23);
       }
       store_split_chunk(h1t[0] + (c >> 3) * RT_TILE, h1t[1] + (c >> 3) * RT_TILE, tid, c & 7, hv);
     }
@@ -188,13 +188,15 @@ __global__ void __launch_bounds__(RT_S, RtCfg<H>::CTAS) rollout_tc_kernel(Rollou
       uint32_t zr[16];
       tc::tmem_ld16(tm_z + lane_base + 16 * c, zr);
       float h2[16];
+      const float2 prescale2 = make_float2(TANH_PRESCALE, TANH_PRESCALE);
 #pragma unroll
       for (int g = 0; g < 4; ++g) {
         const float4 b = lds4(sw + RS_B2 + 16 * c + 4 * g);
-        h2[4 * g] = tanh_prescaled(fmaf(__uint_as_float(zr[4 * g]), TANH_PRESCALE, b.x));
-        h2[4 * g + 1] = tanh_prescaled(fmaf(__uint_as_float(zr[4 * g + 1]), TANH_PRESCALE, b.y));
-        h2[4 * g + 2] = tanh_prescaled(fmaf(__uint_as_float(zr[4 * g + 2]), TANH_PRESCALE, b.z));
-        h2[4 * g + 3] = tanh_prescaled(fmaf(__uint_as_float(zr[4 * g + 3]), TANH_PRESCALE, b.w));
+        const float2 t01 = tanh_prescaled2(__ffma2_rn(make_float2(__uint_as_float(zr[4 * g]), __uint_as_float(zr[4 * g + 1])),
+                                                      prescale2, make_float2(b.x, b.y)));
+        const float2 t23 = tanh_prescaled2(__ffma2_rn(make_float2(__uint_as_float(zr[4 * g + 2]), __uint_as_float(zr[4 * g + 3])),
+                                                      prescale2, make_float2(b.z, b.w)));
+        h2[4 * g] = t01.x; h2[4 * g + 1] = t01.y; h2[4 * g + 2] = t23.x; h2[4 * g + 3] = t23.y;
       }
 #pragma unroll
       for (int k = 0; k < POL_OUT_MAX; ++k) {

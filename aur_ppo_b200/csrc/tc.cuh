@@ -123,12 +123,28 @@ __device__ __forceinline__ void tmem_ld8_nowait(uint32_t taddr, float (&v)[8]) {
 #pragma unroll
   for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
 }
+// the same as 4 column pairs (column 2 i -> v[i].x, 2 i + 1 -> v[i].y), for packed fp32x2 arithmetic
+__device__ __forceinline__ void tmem_ld8_nowait(uint32_t taddr, float2* v) {
+  uint32_t r[8];
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+               : "r"(taddr)
+               : "memory");
+#pragma unroll
+  for (int i = 0; i < 4; ++i) v[i] = make_float2(__uint_as_float(r[2 * i]), __uint_as_float(r[2 * i + 1]));
+}
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 // registers -> TMEM, 32 lanes x 8 columns
 __device__ __forceinline__ void tmem_st8(uint32_t taddr, const float (&v)[8]) {
   asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr),
                "r"(__float_as_uint(v[0])), "r"(__float_as_uint(v[1])), "r"(__float_as_uint(v[2])), "r"(__float_as_uint(v[3])),
                "r"(__float_as_uint(v[4])), "r"(__float_as_uint(v[5])), "r"(__float_as_uint(v[6])), "r"(__float_as_uint(v[7]))
+               : "memory");
+}
+__device__ __forceinline__ void tmem_st8(uint32_t taddr, const float2* v) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr),
+               "r"(__float_as_uint(v[0].x)), "r"(__float_as_uint(v[0].y)), "r"(__float_as_uint(v[1].x)), "r"(__float_as_uint(v[1].y)),
+               "r"(__float_as_uint(v[2].x)), "r"(__float_as_uint(v[2].y)), "r"(__float_as_uint(v[3].x)), "r"(__float_as_uint(v[3].y))
                : "memory");
 }
 // one column: a 32-bit word per lane

@@ -5,16 +5,20 @@
 
 namespace aur {
 
-// 8 fp32 values -> one 16-B chunk of bf16 hi and one of bf16 mid (v - hi), chunk `c` of row `r` (128-B swizzle)
-__device__ __forceinline__ void store_split_chunk(unsigned char* tile_hi, unsigned char* tile_mid, int r, int c, const float* v) {
+// the two bf16 halves of a packed pair, negated, as fp32: adding them takes both residuals with one FADD2
+__device__ __forceinline__ float2 neg_bf16x2(unsigned int w) {
+  return make_float2(-__uint_as_float(w << 16), -__uint_as_float(w & 0xFFFF0000u));
+}
+
+// 8 fp32 values (4 pairs) -> one 16-B chunk of bf16 hi and one of bf16 mid (v - hi), chunk `c` of row `r` (128-B swizzle)
+__device__ __forceinline__ void store_split_chunk(unsigned char* tile_hi, unsigned char* tile_mid, int r, int c, const float2* v) {
   unsigned int hi[4], mid[4];
 #pragma unroll
   for (int e = 0; e < 4; ++e) {
-    const float a = v[2 * e], b = v[2 * e + 1];
-    __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+    __nv_bfloat162 h = __float22bfloat162_rn(v[e]);
     const unsigned int hw = *reinterpret_cast<unsigned int*>(&h);
     hi[e] = hw;
-    __nv_bfloat162 m = __floats2bfloat162_rn(a - __uint_as_float(hw << 16), b - __uint_as_float(hw & 0xFFFF0000u));
+    __nv_bfloat162 m = __float22bfloat162_rn(__fadd2_rn(v[e], neg_bf16x2(hw)));
     mid[e] = *reinterpret_cast<unsigned int*>(&m);
   }
   const int off = r * 128 + ((c ^ (r & 7)) << 4);
@@ -24,17 +28,16 @@ __device__ __forceinline__ void store_split_chunk(unsigned char* tile_hi, unsign
 
 // three-term variant (v = hi + mid + lo, residual <= 2^-25 |v|: fp32-equivalent operands)
 __device__ __forceinline__ void store_split3_chunk(unsigned char* tile_hi, unsigned char* tile_mid, unsigned char* tile_lo, int r, int c,
-                                                   const float* v) {
+                                                   const float2* v) {
   unsigned int hi[4], mid[4], lo[4];
 #pragma unroll
   for (int e = 0; e < 4; ++e) {
-    const float a = v[2 * e], b = v[2 * e + 1];
-    __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+    __nv_bfloat162 h = __float22bfloat162_rn(v[e]);
     const unsigned int hw = *reinterpret_cast<unsigned int*>(&h);
-    const float ra = a - __uint_as_float(hw << 16), rb = b - __uint_as_float(hw & 0xFFFF0000u);
-    __nv_bfloat162 m = __floats2bfloat162_rn(ra, rb);
+    const float2 rs = __fadd2_rn(v[e], neg_bf16x2(hw));
+    __nv_bfloat162 m = __float22bfloat162_rn(rs);
     const unsigned int mw = *reinterpret_cast<unsigned int*>(&m);
-    __nv_bfloat162 l = __floats2bfloat162_rn(ra - __uint_as_float(mw << 16), rb - __uint_as_float(mw & 0xFFFF0000u));
+    __nv_bfloat162 l = __float22bfloat162_rn(__fadd2_rn(rs, neg_bf16x2(mw)));
     hi[e] = hw; mid[e] = mw; lo[e] = *reinterpret_cast<unsigned int*>(&l);
   }
   const int off = r * 128 + ((c ^ (r & 7)) << 4);

@@ -59,6 +59,10 @@ enum { BAR_FWD = 0, BAR_AUX = 1, BAR_WG = 2, BAR_FIN = 3 };
 constexpr int T2_TMEM_COLS = 256;           // z / dh 64 (never live together) | dW2 64 | db2 16 | [db1 dW1] 16 | h1 (fp32 copy) 64
 
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
+// d * (1 - h^2) for a pair of features: the gradient through tanh, h = tanh output (FFMA2 + FMUL2)
+__device__ __forceinline__ float2 tanh_grad2(float2 d, float2 h) {
+  return __fmul2_rn(d, __ffma2_rn(make_float2(-h.x, -h.y), h, make_float2(1.0f, 1.0f)));
+}
 
 struct T2Ptrs {
   unsigned char* base;
@@ -96,18 +100,21 @@ __device__ __forceinline__ void mma_over_samples(uint32_t d, uint64_t a_himid, u
 }
 
 // TPS = threads per sample (2 or 4): each owns FPT = 64 / TPS hidden features of its sample.
+// AOUT = act_dim (1 .. POL_OUT_MAX), the actor's head width; the critic's is 1.  A compile-time width leaves no dead head
+// columns or width tests in the loops.  Adjacent features go through packed fp32x2 ops (FFMA2 / FADD2 / FMUL2) as float2
+// pairs; every lane rounds as the scalar op it replaces, in the same order, so the results are those of scalar code.
 // POP: member blockIdx.y of a population (ppo_grad_tc_kernel<TPS, true>): its parameters, index list, moments and partial rows
 // are offset by pop's strides, its coefficients come from pop.hp and live in shared memory (S2_PC); the argument block itself is
 // never modified, so it stays in the constant bank.
-template <bool ACTOR, int TPS, bool POP>
+template <bool ACTOR, int TPS, bool POP, int AOUT>
 __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop, unsigned char* smem_base, int cta, int ncta) {
-  constexpr int THREADS = 128 * TPS, FPT = 64 / TPS, CPT = FPT / 8;
+  constexpr int THREADS = 128 * TPS, FPT = 64 / TPS, CPT = FPT / 8, FP2 = FPT / 2;
   T2Ptrs P;
   P.base = smem_base;
   const int tid = threadIdx.x, warp = tid >> 5;
   const int s = tid & 127, half = tid >> 7, f0 = FPT * half;      // `half`: which feature slice of the sample (0 .. TPS-1)
-  const int obs_dim = a.obs_dim, A = a.act_dim;
-  const int OUT = ACTOR ? A : 1;
+  const int obs_dim = a.obs_dim;
+  constexpr int A = AOUT, OUT = ACTOR ? A : 1;
   const int64_t gA = net_param_count(obs_dim, UPD_H, 2, A), gC = net_param_count(obs_dim, UPD_H, 2, 1);
 
   // ---- one-time setup: barriers, TMEM, weights, aux tiles
@@ -136,9 +143,9 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
       const int j = tid & 63, cq = tid >> 6;
 #pragma unroll 1
       for (int c = CW * cq; c < CW * cq + CW; ++c) {
-        float v[8];
+        float2 v[4];
 #pragma unroll
-        for (int e = 0; e < 8; ++e) v[e] = gW2[j * 64 + 8 * c + e];
+        for (int e = 0; e < 4; ++e) v[e] = make_float2(gW2[j * 64 + 8 * c + 2 * e], gW2[j * 64 + 8 * c + 2 * e + 1]);
         store_split_chunk(P.w2(0), P.w2(1), j, c, v);
       }
     }
@@ -251,7 +258,7 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
   fetch_obs(rown);
 
   // first layer of one tile: this thread's FPT features from the prefetched observation
-  auto first_layer = [&](float (&hv)[FPT]) {
+  auto first_layer = [&](float2 (&hv)[FP2]) {
 #pragma unroll
     for (int g = 0; g < FPT / 4; ++g) {
       const int f = f0 + 4 * g;
@@ -264,14 +271,14 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
         a01 = __ffma2_rn(make_float2(w.x, w.y), xx, a01);
         a23 = __ffma2_rn(make_float2(w.z, w.w), xx, a23);
       }
-      hv[4 * g] = tanh_prescaled(a01.x); hv[4 * g + 1] = tanh_prescaled(a01.y);
-      hv[4 * g + 2] = tanh_prescaled(a23.x); hv[4 * g + 3] = tanh_prescaled(a23.y);
+      hv[2 * g] = tanh_prescaled2(a01);
+      hv[2 * g + 1] = tanh_prescaled2(a23);
     }
   };
   // TPS 2 computes the next tile's first layer ahead of the MMA wait and carries it across the loop edge; TPS 4 has
   // no registers for that (and twice the warps to cover the wait): it computes it right before storing
   constexpr bool H1_AHEAD = TPS == 2;
-  float h1n[FPT];
+  float2 h1n[FP2];
   if (H1_AHEAD) first_layer(h1n);
 
   uint32_t it = 0;
@@ -292,23 +299,20 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
 #pragma unroll
       for (int c = 0; c < CPT; ++c) {
         const uint32_t col = lane_base + (uint32_t)(f0 + 8 * c);
-        float d[8], hp[8];
+        float2 d[4], hp[4];
         tc::tmem_ld8_nowait(tm_dh + col, d);
         tc::tmem_ld8_nowait(tm_h1 + col, hp);
         tc::tmem_wait_ld();
 #pragma unroll
-        for (int e = 0; e < 8; ++e) d[e] *= fmaf(-hp[e], hp[e], 1.0f);
+        for (int e = 0; e < 4; ++e) d[e] = tanh_grad2(d[e], hp[e]);
         store_split_chunk(P.dz(0), P.dz(1), s, CPT * half + c, d);
       }
     }
     if (!H1_AHEAD) first_layer(h1n);
 #pragma unroll
     for (int c = 0; c < CPT; ++c) {
-      store_split_chunk(P.h1(0), P.h1(1), s, CPT * half + c, h1n + 8 * c);
-      float hv[8];
-#pragma unroll
-      for (int e = 0; e < 8; ++e) hv[e] = h1n[8 * c + e];
-      tc::tmem_st8(tm_h1 + lane_base + (uint32_t)(f0 + 8 * c), hv);
+      store_split_chunk(P.h1(0), P.h1(1), s, CPT * half + c, h1n + 4 * c);
+      tc::tmem_st8(tm_h1 + lane_base + (uint32_t)(f0 + 8 * c), h1n + 4 * c);
     }
     tc::tmem_wait_st();
     {
@@ -363,45 +367,38 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
     // ---- second layer, head, loss
     mbar_wait(P.bar(BAR_FWD), ph);
     tc::fence_after_sync();
-    float h2[FPT];
+    float2 h2[FP2];
 #pragma unroll
     for (int c = 0; c < CPT; ++c) {
-      float zc[8];
-      tc::tmem_ld8_nowait(tm_z + lane_base + (uint32_t)(f0 + 8 * c), zc);
+      tc::tmem_ld8_nowait(tm_z + lane_base + (uint32_t)(f0 + 8 * c), h2 + 4 * c);
       tc::tmem_wait_ld();
-#pragma unroll
-      for (int e = 0; e < 8; ++e) h2[8 * c + e] = zc[e];
     }
+    const float2 prescale2 = make_float2(TANH_PRESCALE, TANH_PRESCALE);
 #pragma unroll
     for (int g = 0; g < FPT / 4; ++g) {
       const float4 b = lds4(sw + S2_B2 + f0 + 4 * g);
-      h2[4 * g] = tanh_prescaled(fmaf(h2[4 * g], TANH_PRESCALE, b.x)); h2[4 * g + 1] = tanh_prescaled(fmaf(h2[4 * g + 1], TANH_PRESCALE, b.y));
-      h2[4 * g + 2] = tanh_prescaled(fmaf(h2[4 * g + 2], TANH_PRESCALE, b.z)); h2[4 * g + 3] = tanh_prescaled(fmaf(h2[4 * g + 3], TANH_PRESCALE, b.w));
+      h2[2 * g] = tanh_prescaled2(__ffma2_rn(h2[2 * g], prescale2, make_float2(b.x, b.y)));
+      h2[2 * g + 1] = tanh_prescaled2(__ffma2_rn(h2[2 * g + 1], prescale2, make_float2(b.z, b.w)));
     }
     float outp[POL_OUT_MAX];             // this half's share of the head pre-activations
 #pragma unroll
     for (int k = 0; k < POL_OUT_MAX; ++k) {
       outp[k] = 0.0f;
       if (k < OUT) {
-        float p0 = 0.0f, p1 = 0.0f;
+        float2 p01 = make_float2(0.0f, 0.0f);        // even / odd features
 #pragma unroll
         for (int g = 0; g < FPT / 4; ++g) {
           const float4 w = lds4(sw + S2_W3 + k * 64 + f0 + 4 * g);
-          p0 = fmaf(w.x, h2[4 * g], p0); p1 = fmaf(w.y, h2[4 * g + 1], p1);
-          p0 = fmaf(w.z, h2[4 * g + 2], p0); p1 = fmaf(w.w, h2[4 * g + 3], p1);
+          p01 = __ffma2_rn(make_float2(w.x, w.y), h2[2 * g], p01);
+          p01 = __ffma2_rn(make_float2(w.z, w.w), h2[2 * g + 1], p01);
         }
-        outp[k] = p0 + p1;
+        outp[k] = p01.x + p01.y;
         if (half > 0) stg[((half - 1) * POL_OUT_MAX + k) * T2_LD + s] = outp[k];     // head exchange: [slice - 1][k][sample]
       }
     }
     if (TPS == 4) {                                    // park h2 in its (consumed) z columns across the loss: registers
 #pragma unroll
-      for (int c = 0; c < CPT; ++c) {
-        float hv[8];
-#pragma unroll
-        for (int e = 0; e < 8; ++e) hv[e] = h2[8 * c + e];
-        tc::tmem_st8(tm_z + lane_base + (uint32_t)(f0 + 8 * c), hv);
-      }
+      for (int c = 0; c < CPT; ++c) tc::tmem_st8(tm_z + lane_base + (uint32_t)(f0 + 8 * c), h2 + 4 * c);
       tc::tmem_wait_st();
     }
     __syncthreads();
@@ -505,11 +502,8 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
     if (TPS == 4) {
 #pragma unroll
       for (int c = 0; c < CPT; ++c) {
-        float hv[8];
-        tc::tmem_ld8_nowait(tm_z + lane_base + (uint32_t)(f0 + 8 * c), hv);
+        tc::tmem_ld8_nowait(tm_z + lane_base + (uint32_t)(f0 + 8 * c), h2 + 4 * c);
         tc::tmem_wait_ld();
-#pragma unroll
-        for (int e = 0; e < 8; ++e) h2[8 * c + e] = hv[e];
       }
     }
     float dout[POL_OUT_MAX];
@@ -519,21 +513,18 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
     mbar_wait(P.bar(BAR_AUX), ph);
 #pragma unroll
     for (int c = 0; c < CPT; ++c) {
-      float dz2[8];
+      float2 dz2[4];
 #pragma unroll
-      for (int e = 0; e < 8; ++e) dz2[e] = 0.0f;
+      for (int e = 0; e < 4; ++e) dz2[e] = make_float2(0.0f, 0.0f);
 #pragma unroll
-      for (int k = 0; k < POL_OUT_MAX; ++k) {
-        if (k < OUT) {
-          const float4 wa = lds4(sw + S2_W3 + k * 64 + f0 + 8 * c), wb = lds4(sw + S2_W3 + k * 64 + f0 + 8 * c + 4);
-          dz2[0] = fmaf(wa.x, dout[k], dz2[0]); dz2[1] = fmaf(wa.y, dout[k], dz2[1]);
-          dz2[2] = fmaf(wa.z, dout[k], dz2[2]); dz2[3] = fmaf(wa.w, dout[k], dz2[3]);
-          dz2[4] = fmaf(wb.x, dout[k], dz2[4]); dz2[5] = fmaf(wb.y, dout[k], dz2[5]);
-          dz2[6] = fmaf(wb.z, dout[k], dz2[6]); dz2[7] = fmaf(wb.w, dout[k], dz2[7]);
-        }
+      for (int k = 0; k < OUT; ++k) {
+        const float4 wa = lds4(sw + S2_W3 + k * 64 + f0 + 8 * c), wb = lds4(sw + S2_W3 + k * 64 + f0 + 8 * c + 4);
+        const float2 dk = make_float2(dout[k], dout[k]);
+        dz2[0] = __ffma2_rn(make_float2(wa.x, wa.y), dk, dz2[0]); dz2[1] = __ffma2_rn(make_float2(wa.z, wa.w), dk, dz2[1]);
+        dz2[2] = __ffma2_rn(make_float2(wb.x, wb.y), dk, dz2[2]); dz2[3] = __ffma2_rn(make_float2(wb.z, wb.w), dk, dz2[3]);
       }
 #pragma unroll
-      for (int e = 0; e < 8; ++e) dz2[e] *= fmaf(-h2[8 * c + e], h2[8 * c + e], 1.0f);
+      for (int e = 0; e < 4; ++e) dz2[e] = tanh_grad2(dz2[e], h2[4 * c + e]);
       store_split_chunk(P.dz(0), P.dz(1), s, CPT * half + c, dz2);
     }
     tc::fence_proxy_async();
@@ -564,7 +555,7 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
       auto put = [&](int p) {
         float* patch = patch0 + (p % NPATCH) * (8 * 36);
 #pragma unroll
-        for (int j = 0; j < 8; ++j) patch[j * 36 + lane] = h2[8 * p + j];
+        for (int j = 0; j < 4; ++j) { patch[2 * j * 36 + lane] = h2[4 * p + j].x; patch[(2 * j + 1) * 36 + lane] = h2[4 * p + j].y; }
       };
       put(0);
       __syncwarp();
@@ -577,11 +568,11 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
         for (int k = 0; k < POL_OUT_MAX; ++k) {
           if (k < OUT) {
             const float4 da = lds4(dbase + k * T2_LD), db = lds4(dbase + k * T2_LD + 4);
-            float s0 = ha.x * da.x, s1 = ha.y * da.y;
-            s0 = fmaf(ha.z, da.z, s0); s1 = fmaf(ha.w, da.w, s1);
-            s0 = fmaf(hb.x, db.x, s0); s1 = fmaf(hb.y, db.y, s1);
-            s0 = fmaf(hb.z, db.z, s0); s1 = fmaf(hb.w, db.w, s1);
-            acc_w3[p][k] += s0 + s1;
+            float2 s01 = __fmul2_rn(make_float2(ha.x, ha.y), make_float2(da.x, da.y));      // even / odd samples
+            s01 = __ffma2_rn(make_float2(ha.z, ha.w), make_float2(da.z, da.w), s01);
+            s01 = __ffma2_rn(make_float2(hb.x, hb.y), make_float2(db.x, db.y), s01);
+            s01 = __ffma2_rn(make_float2(hb.z, hb.w), make_float2(db.z, db.w), s01);
+            acc_w3[p][k] += s01.x + s01.y;
             if (p == 0 && half == 0 && jj == k) acc_b3 += ((da.x + da.y) + (da.z + da.w)) + ((db.x + db.y) + (db.z + db.w));
           }
         }
@@ -601,12 +592,12 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
 #pragma unroll
     for (int c = 0; c < CPT; ++c) {
       const uint32_t col = lane_base + (uint32_t)(f0 + 8 * c);
-      float d[8], hp[8];
+      float2 d[4], hp[4];
       tc::tmem_ld8_nowait(tm_dh + col, d);
       tc::tmem_ld8_nowait(tm_h1 + col, hp);
       tc::tmem_wait_ld();
 #pragma unroll
-      for (int e = 0; e < 8; ++e) d[e] *= fmaf(-hp[e], hp[e], 1.0f);
+      for (int e = 0; e < 4; ++e) d[e] = tanh_grad2(d[e], hp[e]);
       store_split_chunk(P.dz(0), P.dz(1), s, CPT * half + c, d);
     }
     tc::fence_proxy_async();
@@ -729,7 +720,7 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
 
 // POP: population form (aur_pop_update_grad), grid (2 c, K): member k = blockIdx.y trains with its own parameters, index
 // list, advantage moments, coefficients and partial rows; an inactive member (target_kl) does nothing.
-template <int TPS, bool POP = false>
+template <int TPS, bool POP, int AOUT>
 __global__ void __launch_bounds__(128 * TPS, 2) ppo_grad_tc_kernel(UpdDev a, PopUpd pop) {
   extern __shared__ unsigned char smem_raw[];
   unsigned char* base = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // pointer arithmetic keeps the shared address space
@@ -737,43 +728,54 @@ __global__ void __launch_bounds__(128 * TPS, 2) ppo_grad_tc_kernel(UpdDev a, Pop
   if constexpr (POP) {
     if (!pop.active[blockIdx.y]) return;               // the whole CTA: a member stopped by its target_kl
   }
-  if ((int)blockIdx.x < ncta) tc_update_net<true, TPS, POP>(a, pop, base, blockIdx.x, ncta);
-  else tc_update_net<false, TPS, POP>(a, pop, base, blockIdx.x - ncta, ncta);
+  if ((int)blockIdx.x < ncta) tc_update_net<true, TPS, POP, AOUT>(a, pop, base, blockIdx.x, ncta);
+  else tc_update_net<false, TPS, POP, AOUT>(a, pop, base, blockIdx.x - ncta, ncta);
 }
 
 size_t ppo_grad_tc_smem_bytes() { return T2_SMEM; }
 
-template <int TPS>
+template <int TPS, bool POP, int AOUT>
 static int tc_attrs() {
-  AUR_CUDA_OK(cudaFuncSetAttribute(ppo_grad_tc_kernel<TPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T2_SMEM));
+  AUR_CUDA_OK(cudaFuncSetAttribute(ppo_grad_tc_kernel<TPS, POP, AOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T2_SMEM));
   // two CTAs per SM need the full shared-memory carve-out
-  AUR_CUDA_OK(cudaFuncSetAttribute(ppo_grad_tc_kernel<TPS>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  AUR_CUDA_OK(cudaFuncSetAttribute(ppo_grad_tc_kernel<TPS, POP, AOUT>, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                   cudaSharedmemCarveoutMaxShared));
+  return 0;
+}
+
+// one launch of the instantiation for act_dim (1 .. POL_OUT_MAX, checked by the caller)
+template <int TPS, bool POP>
+static int launch_tc(const UpdDev& d, const PopUpd& pop, dim3 grid, cudaStream_t s) {
+  static DeviceOnce attr;
+  if (attr.first()) {
+    int rc;
+    if ((rc = tc_attrs<TPS, POP, 1>()) || (rc = tc_attrs<TPS, POP, 2>()) || (rc = tc_attrs<TPS, POP, 3>()) ||
+        (rc = tc_attrs<TPS, POP, 4>()))
+      return rc;
+    attr.done();
+  }
+  static_assert(POL_OUT_MAX == 4, "one instantiation per act_dim");
+  switch (d.act_dim) {
+    case 1: ppo_grad_tc_kernel<TPS, POP, 1><<<grid, 128 * TPS, T2_SMEM, s>>>(d, pop); break;
+    case 2: ppo_grad_tc_kernel<TPS, POP, 2><<<grid, 128 * TPS, T2_SMEM, s>>>(d, pop); break;
+    case 3: ppo_grad_tc_kernel<TPS, POP, 3><<<grid, 128 * TPS, T2_SMEM, s>>>(d, pop); break;
+    default: ppo_grad_tc_kernel<TPS, POP, 4><<<grid, 128 * TPS, T2_SMEM, s>>>(d, pop); break;
+  }
   return 0;
 }
 
 // gx = CTAs per net (partials are [2][gx][UPD_PSTRIDE]); the grid is 2 * gx.  tps = threads per sample (2 or 4).
 int launch_ppo_grad_tc(const UpdDev& d, int gx, int tps, cudaStream_t s) {
-  static DeviceOnce attr;
-  if (attr.first()) {
-    int rc;
-    if ((rc = tc_attrs<2>()) || (rc = tc_attrs<4>())) return rc;
-    attr.done();
-  }
-  if (tps == 4) ppo_grad_tc_kernel<4><<<2 * gx, 512, T2_SMEM, s>>>(d, PopUpd{});
-  else ppo_grad_tc_kernel<2><<<2 * gx, 256, T2_SMEM, s>>>(d, PopUpd{});
+  const int rc = tps == 4 ? launch_tc<4, false>(d, PopUpd{}, dim3(2 * gx), s) : launch_tc<2, false>(d, PopUpd{}, dim3(2 * gx), s);
+  if (rc) return rc;
   AUR_LAUNCH_OK("ppo_grad_tc_kernel");
   return 0;
 }
 
 // population form: gx CTAs per net and member, K members (two threads per sample)
 int launch_ppo_grad_tc_pop(const UpdDev& d, const PopUpd& pop, int gx, int K, cudaStream_t s) {
-  static DeviceOnce attr;
-  if (attr.first()) {
-    AUR_CUDA_OK(cudaFuncSetAttribute(ppo_grad_tc_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T2_SMEM));
-    AUR_CUDA_OK(cudaFuncSetAttribute(ppo_grad_tc_kernel<2, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    attr.done();
-  }
-  ppo_grad_tc_kernel<2, true><<<dim3(2 * gx, K), 256, T2_SMEM, s>>>(d, pop);
+  const int rc = launch_tc<2, true>(d, pop, dim3(2 * gx, K), s);
+  if (rc) return rc;
   AUR_LAUNCH_OK("ppo_grad_tc_kernel (population)");
   return 0;
 }

@@ -68,9 +68,9 @@ __global__ void __launch_bounds__(VT_THREADS, VtCfg<H>::CTAS) critic_values_tc_k
 #pragma unroll 1
     for (int e = tid; e < H * (H / 8); e += VT_THREADS) {
       const int j = e % H, ch = e / H;
-      float v[8];
+      float2 v[4];
 #pragma unroll
-      for (int q = 0; q < 8; ++q) v[q] = gW2[j * H + 8 * ch + q];
+      for (int q = 0; q < 4; ++q) v[q] = make_float2(gW2[j * H + 8 * ch + 2 * q], gW2[j * H + 8 * ch + 2 * q + 1]);
       const int o = (ch >> 3) * Cfg::WTILE;
       store_split3_chunk(w2t[0] + o, w2t[1] + o, w2t[2] + o, j, ch & 7, v);
     }
@@ -117,7 +117,7 @@ __global__ void __launch_bounds__(VT_THREADS, VtCfg<H>::CTAS) critic_values_tc_k
     // ---- first layer -> operand rows (8-feature chunks)
 #pragma unroll
     for (int c = 0; c < FPT / 8; ++c) {
-      float hv[8];
+      float2 hv[4];
 #pragma unroll
       for (int g = 0; g < 2; ++g) {
         const int f = f0 + 8 * c + 4 * g;
@@ -130,8 +130,8 @@ __global__ void __launch_bounds__(VT_THREADS, VtCfg<H>::CTAS) critic_values_tc_k
           a01 = __ffma2_rn(make_float2(w.x, w.y), xx, a01);
           a23 = __ffma2_rn(make_float2(w.z, w.w), xx, a23);
         }
-        hv[4 * g] = tanh_prescaled(a01.x); hv[4 * g + 1] = tanh_prescaled(a01.y);
-        hv[4 * g + 2] = tanh_prescaled(a23.x); hv[4 * g + 3] = tanh_prescaled(a23.y);
+        hv[2 * g] = tanh_prescaled2(a01);
+        hv[2 * g + 1] = tanh_prescaled2(a23);
       }
       const int ch = (FPT / 8) * half + c, o = (ch >> 3) * VT_TILE;
       store_split3_chunk(h1t[0] + o, h1t[1] + o, h1t[2] + o, s, ch & 7, hv);
@@ -154,7 +154,8 @@ __global__ void __launch_bounds__(VT_THREADS, VtCfg<H>::CTAS) critic_values_tc_k
     load_obs(tile + gridDim.x, xn);                  // next tile's rows, in flight across the MMA round trip
     mbar_wait(bar, it & 1u);
     tc::fence_after_sync();
-    float p0 = 0.0f, p1 = 0.0f;
+    float2 p01 = make_float2(0.0f, 0.0f);            // even / odd features
+    const float2 prescale2 = make_float2(TANH_PRESCALE, TANH_PRESCALE);
 #pragma unroll
     for (int q = 0; q < FPT / 32; ++q) {
       float z[32];
@@ -162,12 +163,11 @@ __global__ void __launch_bounds__(VT_THREADS, VtCfg<H>::CTAS) critic_values_tc_k
 #pragma unroll
       for (int g = 0; g < 8; ++g) {
         const float4 b = lds4(sw + VS_B2 + f0 + 32 * q + 4 * g), w = lds4(sw + VS_W3 + f0 + 32 * q + 4 * g);
-        p0 = fmaf(w.x, tanh_prescaled(fmaf(z[4 * g], TANH_PRESCALE, b.x)), p0);
-        p1 = fmaf(w.y, tanh_prescaled(fmaf(z[4 * g + 1], TANH_PRESCALE, b.y)), p1);
-        p0 = fmaf(w.z, tanh_prescaled(fmaf(z[4 * g + 2], TANH_PRESCALE, b.z)), p0);
-        p1 = fmaf(w.w, tanh_prescaled(fmaf(z[4 * g + 3], TANH_PRESCALE, b.w)), p1);
+        p01 = __ffma2_rn(make_float2(w.x, w.y), tanh_prescaled2(__ffma2_rn(make_float2(z[4 * g], z[4 * g + 1]), prescale2, make_float2(b.x, b.y))), p01);
+        p01 = __ffma2_rn(make_float2(w.z, w.w), tanh_prescaled2(__ffma2_rn(make_float2(z[4 * g + 2], z[4 * g + 3]), prescale2, make_float2(b.z, b.w))), p01);
       }
     }
+    const float p0 = p01.x, p1 = p01.y;
     // the upper half hands its head partial over through a TMEM column of its own (already consumed) z range
     if (half == 1) { tc::tmem_st1(tm_z + lane_base + FPT, p0 + p1); tc::tmem_wait_st(); }
     tc::fence_before_sync();
