@@ -279,14 +279,18 @@ __device__ __forceinline__ void categorical(const float (&logits)[POL_OUT_MAX], 
     if (k < A) entropy -= pr[k] * lp[k];
   }
   if (sample) {
+    // the fp32 running sum can end a few ulp below 1, under the largest u (1 - 2^-24): such a draw takes the last class
+    // with nonzero probability, never one whose probability underflowed to 0
     float c = 0.0f;
-    action = A - 1;
+    int last = 0;
     bool found = false;
 #pragma unroll
     for (int k = 0; k < POL_OUT_MAX; ++k) {
       c += pr[k];
+      if (k < A && pr[k] > 0.0f) last = k;
       if (k < A && !found && u < c) { action = k; found = true; }
     }
+    if (!found) action = last;
   }
   logp = lp[0];
 #pragma unroll

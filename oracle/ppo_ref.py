@@ -17,7 +17,9 @@ the library the reference itself computes with.
   explained_variance       ppo.py:277-279
   lr_anneal                ppo.py:195-198
   philox4x32_10 / sampling the device sampler's counter-based stream, restated
-                           so sampled rollouts can be replayed on the CPU
+                           so sampled rollouts can be replayed on the CPU; the
+                           vectorised forms and normal4_f64 / categorical_icdf
+                           restate every draw in float64
 """
 from __future__ import annotations
 
@@ -240,6 +242,62 @@ def sampler_words(seed: int, env_id: int, step: int) -> Tuple[int, int, int, int
 def u01(word: int) -> np.float32:
     """24-bit uniform in [0,1): (w >> 8) * 2^-24."""
     return np.float32((word >> 8) * (1.0 / 16777216.0))
+
+
+# Vectorised forms of the above, for checking every draw of a launch.  Each device sampler keys one Philox4x32-10 block
+# by the 64-bit seed and builds its counter from two 64-bit ids and a dimension block (dims 4 blk .. 4 blk + 3):
+#   rollouts, policy_evaluate:     (gid lo, gid hi, step lo, step hi ^ blk << 24)   gid = env_id0 + env or row0 + row
+#   aur_squashed_gaussian_sample:  (row lo, row hi, stream lo, stream hi ^ blk << 24)
+#   head_eval_kernel (facades):    (b, 0, stream lo, stream hi ^ blk << 24)          b < 2^31, so b hi = 0
+_U32 = np.uint64(0xFFFFFFFF)
+
+
+def philox4x32_10_np(c0, c1, c2, c3, k0, k1) -> np.ndarray:
+    """philox4x32_10 over broadcast arrays of counter and key words -> uint32 [4, ...] (words c[0..3])."""
+    c0, c1, c2, c3, k0, k1 = np.broadcast_arrays(*[np.asarray(x, dtype=np.uint64) & _U32 for x in (c0, c1, c2, c3, k0, k1)])
+    k0, k1 = k0.copy(), k1.copy()
+    m0, m1, w0, w1, s32 = np.uint64(_M0), np.uint64(_M1), np.uint64(_W0), np.uint64(_W1), np.uint64(32)
+    for _ in range(10):
+        p0, p1 = c0 * m0, c2 * m1
+        c0, c1, c2, c3 = (p1 >> s32) ^ c1 ^ k0, p1 & _U32, (p0 >> s32) ^ c3 ^ k1, p0 & _U32
+        k0 = (k0 + w0) & _U32
+        k1 = (k1 + w1) & _U32
+    return np.stack([c0, c1, c2, c3]).astype(np.uint32)
+
+
+def sampler_counter(idx, stream, blk: int = 0):
+    """The four counter words (idx lo, idx hi, stream lo, stream hi ^ blk << 24) of the table above."""
+    idx, stream = np.asarray(idx, dtype=np.uint64), np.asarray(stream, dtype=np.uint64)
+    return idx & _U32, idx >> np.uint64(32), stream & _U32, (stream >> np.uint64(32)) ^ np.uint64(blk << 24)
+
+
+def sampler_words_np(seed: int, idx, stream, blk: int = 0) -> np.ndarray:
+    """uint32 [4, ...]: the Philox block a device sampler draws for (idx, stream, dimension block blk) under `seed`."""
+    return philox4x32_10_np(*sampler_counter(idx, stream, blk), seed & 0xFFFFFFFF, (seed >> 32) & 0xFFFFFFFF)
+
+
+def normal4_f64(words: np.ndarray) -> np.ndarray:
+    """Box-Muller of policy.cuh normal4 in float64: u = ((w >> 8) + 1/2) 2^-24 lies in (0, 1) for every word, and
+    z = sqrt(-2 ln u1) (cos, sin)(2 pi u2), sqrt(-2 ln u3) (cos, sin)(2 pi u4).  words [4, ...] -> z [..., 4]."""
+    u = ((np.asarray(words, dtype=np.uint32) >> np.uint32(8)).astype(np.float64) + 0.5) * 2.0 ** -24
+    ra, rb = np.sqrt(-2.0 * np.log(u[0])), np.sqrt(-2.0 * np.log(u[2]))
+    return np.stack([ra * np.cos(2 * np.pi * u[1]), ra * np.sin(2 * np.pi * u[1]),
+                     rb * np.cos(2 * np.pi * u[3]), rb * np.sin(2 * np.pi * u[3])], axis=-1)
+
+
+def categorical_icdf(probs, u):
+    """Inverse CDF of Categorical(probs): the first class k with u < P_0 + .. + P_k; a u at or past the total takes the last
+    class with nonzero probability.  probs [n, A] float64, u [n] -> (class [n] int64, distance of u to the nearest interior
+    CDF boundary [n]; inf when A = 1), so that a check can leave out draws closer to a boundary than a kernel's error."""
+    probs = np.asarray(probs, dtype=np.float64)
+    u = np.asarray(u, dtype=np.float64)
+    cdf = np.cumsum(probs, axis=1)
+    cls = (cdf <= u[:, None]).sum(axis=1)
+    last_nz = probs.shape[1] - 1 - np.argmax(probs[:, ::-1] > 0, axis=1)
+    cls = np.where(cls >= probs.shape[1], last_nz, cls)
+    inner = cdf[:, :-1]
+    margin = np.abs(inner - u[:, None]).min(axis=1) if inner.shape[1] else np.full(u.shape, np.inf)
+    return cls.astype(np.int64), margin
 
 
 # ------------------------------------------------- device minibatch shuffle, restated on CPU
