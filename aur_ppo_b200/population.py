@@ -30,7 +30,7 @@ from typing import Dict, List, Optional, Sequence
 import numpy as np
 import torch
 
-from . import _lib, compat, kernels, parallel
+from . import _lib, compat, kernels, parallel, state
 from .envs import DeviceVecEnv, pcg64_seed_states
 from .models.actor_critic import actor_critic
 from .ppo import _SPACES, torch_buffer
@@ -185,6 +185,9 @@ class ppo_population:
         self.pop = _lib.PopDesc(K, 0, self.n_member, self.seeds.data_ptr())
         self.bias_corr = None
         self._iterations = 0
+        self._iteration = 0              # iterations of train() completed
+        self._train_seconds = 0.0        # wall-clock seconds train() has run them in
+        self._resumed = False            # load_state() restored a state: the next train() continues it
         self._ensure_bias_corr(self.num_updates * self.n_mb + 1)
 
         # ---- envs, buffers, workspace
@@ -232,6 +235,64 @@ class ppo_population:
             bc[s, 0] = 1.0 - math.pow(ADAM_BETAS[0], float(s))
             bc[s, 1] = 1.0 - math.pow(ADAM_BETAS[1], float(s))
         self.bias_corr = torch.from_numpy(bc).to(self.device)
+
+    # ------------------------------------------------------------------ training state
+    def _state_fingerprint(self) -> Dict:
+        return state.fingerprint(self.params_dict, self.members, self.pbt)
+
+    def _state_tensors(self) -> Dict[str, torch.Tensor]:
+        out = dict(params=self.params, exp_avg=self.exp_avg, exp_avg_sq=self.exp_avg_sq, steps=self.steps,
+                   hparams=self.hparams, totals=self.totals)
+        if self.pbt is not None:
+            out["pbt_snapshot"] = self.pbt_snapshot
+        return out
+
+    def save_state(self, path: str) -> None:
+        """Write what train() needs to continue after iteration `self._iteration` to `path` (state.py, DESIGN.md section 13)."""
+        if self._iteration < 1:
+            raise _lib.AurError("save_state: no iteration of train() has completed yet; there is nothing to resume")
+        body = dict(tensors=state.to_host(self._state_tensors()), env=state.to_host(state.env_tensors(self.envs)),
+                    env_step=int(self._env_step), shuffle_count=int(self._shuffle_count), iterations=int(self._iterations),
+                    iteration=int(self._iteration), train_seconds=float(self._train_seconds), run_name=self.run_name,
+                    member_params=[{key: mp[key] for key in SWEEP_KEYS} for mp in self.member_params],
+                    any_target_kl=bool(self.any_target_kl),
+                    total_returns=[state.history(r, np.float64) for r in self.total_returns],
+                    total_episode_lengths=[state.history(r, np.int64) for r in self.total_episode_lengths],
+                    x_indices=[state.history(r, np.int64) for r in self.x_indices], pbt_round=int(self.pbt_round),
+                    lineage=list(self.lineage))
+        state.write(path, "population", self._state_fingerprint(), body)
+
+    def load_state(self, path: str) -> None:
+        """Restore a state written by save_state into this freshly built population (same configuration, members and PBT
+        config); the next train() then continues with the following iteration, without an env reset.  Everything is checked
+        before anything is changed.  Tensors are copied in place: the members' parameters stay views of the [K][P] buffer."""
+        st = state.read(path, "population", self._state_fingerprint())
+        f = state.fields(st, ("tensors", "env", "env_step", "shuffle_count", "iterations", "iteration", "train_seconds",
+                              "run_name", "member_params", "any_target_kl", "total_returns", "total_episode_lengths",
+                              "x_indices", "pbt_round", "lineage"))
+        K = self.K
+        try:
+            v = dict(env_step=int(f["env_step"]), shuffle_count=int(f["shuffle_count"]), iterations=int(f["iterations"]),
+                     iteration=int(f["iteration"]), train_seconds=float(f["train_seconds"]), run_name=str(f["run_name"]),
+                     member_params=[{key: m[key] for key in SWEEP_KEYS} for m in f["member_params"]],
+                     any_target_kl=bool(f["any_target_kl"]), pbt_round=int(f["pbt_round"]), lineage=list(f["lineage"]),
+                     **{key: [t.tolist() for t in f[key]] for key in ("total_returns", "total_episode_lengths", "x_indices")})
+        except (AttributeError, KeyError, TypeError, ValueError) as e:
+            raise _lib.AurError(f"training state {path!r}: malformed entry ({e!r})")
+        if any(len(v[key]) != K for key in ("member_params", "total_returns", "total_episode_lengths", "x_indices")):
+            raise _lib.AurError(f"training state {path!r}: per-member entries do not have {K} members")
+        mine = self._state_tensors()
+        state.restore([(k, t, f["tensors"].get(k)) for k, t in mine.items()] + state.restore_env(self.envs, f["env"]))
+        self._env_step, self._shuffle_count = v["env_step"], v["shuffle_count"]
+        self._iterations, self._iteration = v["iterations"], v["iteration"]
+        self._train_seconds, self.run_name = v["train_seconds"], v["run_name"]
+        self._ensure_bias_corr(self._iterations * self.n_mb)
+        for mp, saved in zip(self.member_params, v["member_params"]):
+            mp.update(saved)
+        self.any_target_kl = v["any_target_kl"]
+        self.total_returns, self.total_episode_lengths, self.x_indices = v["total_returns"], v["total_episode_lengths"], v["x_indices"]
+        self.pbt_round, self.lineage = v["pbt_round"], v["lineage"]
+        self._resumed = True
 
     # ------------------------------------------------------------------ hot path pieces
     def reset_envs(self) -> None:
@@ -377,8 +438,15 @@ class ppo_population:
         """Member k's [T, n_member, ...] part of a [T, K * n_member, ...] population buffer."""
         return t[:, k * self.n_member:(k + 1) * self.n_member]
 
-    def train(self):
-        """ppo.train for every member -> one (total_returns, total_episode_lengths, x_indices) per member."""
+    def train(self, save_state_every: int = 0, state_path: str = "training_state.pt", resume: Optional[str] = None):
+        """ppo.train for every member -> one (total_returns, total_episode_lengths, x_indices) per member.
+        save_state_every N > 0: write the training state to `state_path` after every N-th iteration (after its PBT round) and
+        after the last one.  resume: continue the population whose state that file holds; the same as load_state(resume)
+        followed by train()."""
+        if int(save_state_every) < 0:
+            raise _lib.AurError(f"save_state_every must be >= 0 (got {save_state_every})")
+        if resume is not None:
+            self.load_state(resume)
         K, n, T = self.K, self.n_member, int(self.num_steps)
         writers = [None] * K
         if self.params_dict.get("tensorboard", True):
@@ -388,9 +456,12 @@ class ppo_population:
                 writers[k].add_text("parameters/what", "what")
                 writers[k].add_text("hyperparameters", "|param|value|\n|-|-|\n%s" % (
                     "\n".join([f"|{key}|{str(mp[key])}|" for key in mp])))
-        start_time = time.time()
-        self.reset_envs()
-        for update in range(1, self.num_updates + 1):
+        resuming, self._resumed = self._resumed, False
+        if not resuming:
+            self.reset_envs()
+            self._iteration, self._train_seconds = 0, 0.0
+        start_time = time.time() - self._train_seconds
+        for update in range(self._iteration + 1, self.num_updates + 1):
             step_base = self._env_step
             out = self.run_update(update)
             keys = self.first_finished.cpu().numpy().view(np.uint64)
@@ -437,6 +508,9 @@ class ppo_population:
                         f = entry["fitness"][k]
                         w.add_scalar("pbt/fitness", float("nan") if f is None else f, global_step)
                         w.add_scalar("pbt/donor", entry["donor"][k], global_step)
+            self._iteration, self._train_seconds = update, time.time() - start_time
+            if save_state_every and (update % save_state_every == 0 or update == self.num_updates):
+                self.save_state(state_path)
         for w in writers:
             if w is not None:
                 w.close()

@@ -29,7 +29,7 @@ from typing import Dict, List, Optional
 import numpy as np
 import torch
 
-from . import _lib, compat, kernels, parallel
+from . import _lib, compat, kernels, parallel, state
 from .envs import DeviceVecEnv
 from .models.actor_critic import actor_critic
 
@@ -145,6 +145,9 @@ class ppo:
         self._returns = torch.empty_like(self.buffer.rewards)
         self._advantages = torch.empty_like(self.buffer.rewards)
         self._env_step = 0
+        self._iteration = 0              # iterations of train() completed
+        self._train_seconds = 0.0        # wall-clock seconds train() has run them in
+        self._resumed = False            # load_state() restored a state: the next train() continues it
 
     def close(self) -> None:
         """Unmap the peer exchange areas (data-parallel runs); collective: every rank calls it."""
@@ -237,8 +240,68 @@ class ppo:
         rec(3)
         return dict(stats=stats_rows[:n_mb], b_values=flat_bufs[5], b_returns=flat_bufs[4])
 
+    # --------------------------------------------------------------------------- training state
+    def _state_tensors(self) -> Dict[str, torch.Tensor]:
+        return dict(flat=self.flat, exp_avg=self.updater.exp_avg, exp_avg_sq=self.updater.exp_avg_sq,
+                    totals=self.envs.totals)
+
+    def _refuse_data_parallel(self) -> None:
+        if self.world_size > 1:
+            raise _lib.AurError("training state: data-parallel runs (world_size > 1) cannot be saved or resumed")
+
+    def save_state(self, path: str) -> None:
+        """Write what train() needs to continue after iteration `self._iteration` to `path` (state.py, DESIGN.md section 13)."""
+        self._refuse_data_parallel()
+        if self._iteration < 1:
+            raise _lib.AurError("save_state: no iteration of train() has completed yet; there is nothing to resume")
+        body = dict(tensors=state.to_host(self._state_tensors()), env=state.to_host(state.env_tensors(self.envs)),
+                    step_count=int(self.updater.step_count), env_step=int(self._env_step),
+                    shuffle_count=int(self._shuffle_count), iteration=int(self._iteration),
+                    train_seconds=float(self._train_seconds), run_name=self.run_name,
+                    total_returns=state.history(self.total_returns, np.float64),
+                    total_episode_lengths=state.history(self.total_episode_lengths, np.int64),
+                    x_indices=state.history(self.x_indices, np.int64), last_stats=getattr(self, "last_stats", None))
+        state.write(path, "ppo", state.fingerprint(self.params_dict), body)
+
+    def load_state(self, path: str) -> None:
+        """Restore a state written by save_state into this freshly built run (same configuration); the next train() then
+        continues with the following iteration, without an env reset.  Everything is checked before anything is changed.
+        Tensors are copied in place: `flat` stays the buffer the policy's parameters view."""
+        self._refuse_data_parallel()
+        st = state.read(path, "ppo", state.fingerprint(self.params_dict))
+        f = state.fields(st, ("tensors", "env", "step_count", "env_step", "shuffle_count", "iteration", "train_seconds",
+                              "run_name", "total_returns", "total_episode_lengths", "x_indices", "last_stats"))
+        try:
+            scalars = dict(step_count=int(f["step_count"]), env_step=int(f["env_step"]), shuffle_count=int(f["shuffle_count"]),
+                           iteration=int(f["iteration"]), train_seconds=float(f["train_seconds"]), run_name=str(f["run_name"]),
+                           total_returns=f["total_returns"].tolist(), total_episode_lengths=f["total_episode_lengths"].tolist(),
+                           x_indices=f["x_indices"].tolist(), last_stats=None if f["last_stats"] is None else dict(f["last_stats"]))
+        except (AttributeError, TypeError, ValueError) as e:
+            raise _lib.AurError(f"training state {path!r}: malformed entry ({e})")
+        mine = self._state_tensors()
+        state.restore([(k, t, f["tensors"].get(k)) for k, t in mine.items()] + state.restore_env(self.envs, f["env"]))
+        self.updater.step_count = scalars["step_count"]
+        self._env_step, self._shuffle_count = scalars["env_step"], scalars["shuffle_count"]
+        self._iteration, self._train_seconds = scalars["iteration"], scalars["train_seconds"]
+        self.run_name = scalars["run_name"]
+        self.total_returns = scalars["total_returns"]
+        self.total_episode_lengths = scalars["total_episode_lengths"]
+        self.x_indices = scalars["x_indices"]
+        if scalars["last_stats"] is not None:
+            self.last_stats = scalars["last_stats"]
+        self._resumed = True
+
     # --------------------------------------------------------------------------- train
-    def train(self):
+    def train(self, save_state_every: int = 0, state_path: str = "training_state.pt", resume: Optional[str] = None):
+        """ppo.py:175-309.  save_state_every N > 0: write the training state to `state_path` after every N-th iteration and
+        after the last one.  resume: continue the run whose state that file holds (no env reset, same schedule); the same as
+        load_state(resume) followed by train()."""
+        if int(save_state_every) < 0:
+            raise _lib.AurError(f"save_state_every must be >= 0 (got {save_state_every})")
+        if save_state_every or resume is not None:
+            self._refuse_data_parallel()
+        if resume is not None:
+            self.load_state(resume)
         writer = None
         if self.rank == 0 and self.params_dict.get("tensorboard", True):
             if self.track:
@@ -256,13 +319,16 @@ class ppo:
         torch.manual_seed(seed)
 
         global_step = 0
-        start_time = time.time()
-        self.envs.reset(seed=list(self.plan.env_ids))
-        self._env_step = 0
+        resuming, self._resumed = self._resumed, False
+        if not resuming:
+            self.envs.reset(seed=list(self.plan.env_ids))
+            self._env_step = 0
+            self._iteration, self._train_seconds = 0, 0.0
+        start_time = time.time() - self._train_seconds
         n_rows = self.num_update_epochs * math.ceil(self.local_batch / max(self.local_minibatch, 1))
         self._stats_rows = torch.zeros(n_rows, kernels.NUM_STATS, device=self.device)
 
-        for update in range(1, self.num_updates + 1):
+        for update in range(self._iteration + 1, self.num_updates + 1):
             step_base = self._env_step
             out = self.run_update(update)
             self._check_exchange()
@@ -297,6 +363,9 @@ class ppo:
                 writer.add_scalar("losses/clipfrac", host[8], global_step)
                 writer.add_scalar("losses/explained_variance", explained_var, global_step)
                 writer.add_scalar("charts/SPS", int(global_step / (time.time() - start_time)), global_step)
+            self._iteration, self._train_seconds = update, time.time() - start_time
+            if save_state_every and (update % save_state_every == 0 or update == self.num_updates):
+                self.save_state(state_path)
 
         self.envs.close()
         self.close()

@@ -15,6 +15,10 @@ Additions (all opt-in, none changes a reference default):
   --pbt_fraction Q           the share of members that copy, and that are copied from, each round (0 < Q <= 0.5; 0.25)
   --pbt_keys K1,K2           the hyper-parameters a copy perturbs by x0.8 or x1.2 (per-member keys above;
                              learning_rate,entropy_coeff)
+  --save_state_every N       write the training state (weights, Adam moments, env and RNG counters, episode history; state.py)
+                             to training_state.pt every N iterations and after the last one (0 = off, the default)
+  --resume PATH              continue the run whose training state PATH holds, bit for bit as if it had not stopped; the
+                             other flags must describe the same run (a differing setting is refused by name)
 """
 from __future__ import annotations
 
@@ -75,6 +79,9 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument('--pbt_interval', type=int, default=0, help='population-based training every N iterations (0 = off)')
     p.add_argument('--pbt_fraction', type=float, default=0.25, help='share of members replaced per PBT round, in (0, 0.5]')
     p.add_argument('--pbt_keys', type=str, default='learning_rate,entropy_coeff', help='hyper-parameters a PBT copy perturbs')
+    p.add_argument('--save_state_every', type=int, default=0,
+                   help='write training_state.pt every N iterations and after the last one (0 = off)')
+    p.add_argument('--resume', type=str, default=None, metavar='PATH', help='continue the run whose training state PATH holds')
     return p
 
 
@@ -165,12 +172,15 @@ def main(argv: Optional[List[str]] = None):
         pbt = pbt_from_args(args, len(members))
     except ValueError as e:
         parser.error(str(e))
+    if args.save_state_every < 0:
+        parser.error("--save_state_every must be >= 0")
+    state_args = dict(save_state_every=args.save_state_every, resume=args.resume)
     if members:
         from .population import ppo_population
-        return ppo_population(params, members, pbt=pbt).train()
+        return ppo_population(params, members, pbt=pbt).train(**state_args)
     from .ppo import ppo
     to_run = ppo(params)
-    return to_run.train()
+    return to_run.train(**state_args)
 
 
 if __name__ == '__main__':
