@@ -6,7 +6,8 @@ Imported only by tests/, __graft_entry__.smoke() and bench.py's cpu_baseline /
 Pinned: every function here is checked against tests/golden/*.npz, which
 oracle/gen_golden.py produced by running the reference's own code
 (tests/test_oracle_ppo.py).  Floating point work uses torch fp32 on the CPU,
-the library the reference itself computes with.
+the library the reference itself computes with; RefPolicy(dtype=torch.float64)
+runs the same update in float64.
 
   gae / normal_advantage   ppo.py:125-142 / ppo.py:145-157
   MLP forward              nets/nets.py:19-53 (Linear-Tanh stacks)
@@ -68,10 +69,12 @@ def normal_advantage(rewards, values, terminals, next_value, next_done, gamma: f
 # ------------------------------------------------------------------------- model
 class RefPolicy:
     """Parameter container in the reference's naming: actor.net.{0,2,..}.{weight,bias},
-    critic.net.{...}, optional actor_logstd [1,A] (models/actor_critic.py:8-26)."""
+    critic.net.{...}, optional actor_logstd [1,A] (models/actor_critic.py:8-26).
+    dtype: float32 is the reference's own arithmetic; float64 gives the high-precision value that the fp32 kernels and the
+    fp32 restatement are both measured against (ppo_loss, clip_grad_norm and RefAdam follow the parameters' dtype)."""
 
-    def __init__(self, params: Dict[str, torch.Tensor], continuous: bool):
-        self.p = {k: (v if isinstance(v, torch.Tensor) else torch.from_numpy(np.asarray(v))).clone().float()
+    def __init__(self, params: Dict[str, torch.Tensor], continuous: bool, dtype: torch.dtype = torch.float32):
+        self.p = {k: (v if isinstance(v, torch.Tensor) else torch.from_numpy(np.asarray(v))).clone().to(dtype)
                   for k, v in params.items()}
         self.continuous = continuous
 
@@ -100,7 +103,7 @@ class RefPolicy:
             logstd = self.p["actor_logstd"].expand_as(head)
             std = torch.exp(logstd)
             if action is None:
-                action = head + std * torch.randn(head.shape, generator=generator)
+                action = head + std * torch.randn(head.shape, generator=generator, dtype=head.dtype)
                 action = action.detach()
             var = std ** 2
             log_scale = std.log()      # torch Normal: log(exp(logstd)), not logstd itself
@@ -138,7 +141,7 @@ def ppo_loss(policy: RefPolicy, obs, act, oldlp, adv, ret, vold, clip_coeff=0.2,
     with torch.no_grad():
         old_approx_kl = (-log_ratio).mean()
         approx_kl = ((ratio - 1) - log_ratio).mean()
-        clipfrac = ((ratio - 1.0).abs() > clip_coeff).float().mean()
+        clipfrac = ((ratio - 1.0).abs() > clip_coeff).to(ratio.dtype).mean()
     mb_adv = adv
     if norm_adv:
         mb_adv = (mb_adv - mb_adv.mean()) / (mb_adv.std() + 1e-8)

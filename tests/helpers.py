@@ -5,7 +5,7 @@ import torch
 from oracle import ppo_ref as R
 
 
-def flat_from_named(named: dict) -> np.ndarray:
+def flat_from_named(named: dict, dtype=np.float32) -> np.ndarray:
     """Canonical flat parameter order of include/aur_ppo.h from the reference's names."""
     def net(prefix):
         idx = sorted({int(k.split(".")[2]) for k in named if k.startswith(prefix + ".net.")})
@@ -16,7 +16,7 @@ def flat_from_named(named: dict) -> np.ndarray:
     parts = net("actor") + net("critic")
     if "actor_logstd" in named:
         parts.append(np.asarray(named["actor_logstd"]).ravel())
-    return np.concatenate(parts).astype(np.float32)
+    return np.concatenate(parts).astype(dtype)
 
 
 def golden_policy(golden_dir, tag, file="model.npz", prefix="p"):

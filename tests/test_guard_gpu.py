@@ -47,12 +47,24 @@ def test_gae_writes_stay_inside(T, N):
     ret.check("returns", True); adv.check("advantages", True)
 
 
-@pytest.mark.parametrize("gym_id,cont,act,N,T", [("CartPole-v1", False, 2, 130, 9), ("CartPole-v1", False, 2, 9600, 5),
-                                                   ("Pendulum-v1", True, 1, 257, 7), ("Acrobot-v1", False, 3, 100, 6)])
-def test_rollout_writes_stay_inside(gym_id, cont, act, N, T):
+# gym_id, continuous, act_dim, N, T, hidden.  The wide rows are the first guarded runs of the layer-wise actor with the
+# external-actor env step (CartPole 256 x 2) and of rollout_tc_kernel<ENV, 128> + critic_values_tc_kernel<128> (Pendulum and
+# MountainCar 128 x 2); under impl 0 they run the runtime-width SIMT kernel
+ROLLOUT_GUARDS = {"CartPole-v1-False-2-130-9": ("CartPole-v1", False, 2, 130, 9, 64),
+                  "CartPole-v1-False-2-9600-5": ("CartPole-v1", False, 2, 9600, 5, 64),
+                  "Pendulum-v1-True-1-257-7": ("Pendulum-v1", True, 1, 257, 7, 64),
+                  "Acrobot-v1-False-3-100-6": ("Acrobot-v1", False, 3, 100, 6, 64),
+                  "cartpole-256x2": ("CartPole-v1", False, 2, 130, 5, 256),
+                  "pendulum-128x2": ("Pendulum-v1", True, 1, 257, 7, 128),
+                  "mountaincar-128x2": ("MountainCar-v0", False, 3, 300, 6, 128)}
+
+
+@pytest.mark.parametrize("case", list(ROLLOUT_GUARDS))
+def test_rollout_writes_stay_inside(case):
+    gym_id, cont, act, N, T, hidden = ROLLOUT_GUARDS[case]
     env = denv.DeviceVecEnv(gym_id, N, wrappers=cont)
     env.reset(list(range(N)))
-    desc = kernels.policy_desc(env.obs_dim, act, 64, 2, cont)
+    desc = kernels.policy_desc(env.obs_dim, act, hidden, 2, cont)
     P = kernels.policy_param_count(desc)
     flat = (torch.rand(P, device="cuda") - 0.5) * 0.2
     buf = kernels.RolloutBuffers(T, N, env.obs_dim, (act,) if cont else (), "cuda")
@@ -70,12 +82,23 @@ def test_rollout_writes_stay_inside(gym_id, cont, act, N, T):
     _lib.lib().aur_rollout_set_impl(1)
 
 
+# continuous, m, hidden, layers.  The wide rows are the first guarded runs of the layer-wise update (update_wide.cu): m = 65
+# ends one sample into the second 64-sample TMA box, m = 1025 one sample into the second 1,024-sample partial row; 256 x 3 adds
+# the middle layer.  They take that path whatever the impl switch says, so they run once.
+UPDATE_GUARDS = {"False-1000": (False, 1000, 64, 2), "True-129": (True, 129, 64, 2), "False-4097": (False, 4097, 64, 2)}
+UPDATE_GUARDS.update({f"{'cont' if c else 'disc'}{h}x{nl}-{m}": (c, m, h, nl) for h, nl in ((128, 2), (256, 3))
+                      for c in (False, True) for m in (65, 1025)})
+
+
 @pytest.mark.parametrize("impl", [0, 1, 2, 3])
-@pytest.mark.parametrize("cont,m", [(False, 1000), (True, 129), (False, 4097)])
-def test_update_writes_stay_inside(impl, cont, m):
+@pytest.mark.parametrize("case", list(UPDATE_GUARDS))
+def test_update_writes_stay_inside(impl, case):
+    cont, m, hidden, layers = UPDATE_GUARDS[case]
+    if hidden != 64 and impl != 1:
+        pytest.skip("one kernel behind this shape")
     obs_dim, act_dim = (3, 1) if cont else (4, 2)
-    _, named = random_policy(obs_dim, act_dim, 64, 2, cont, seed=4)
-    desc = kernels.policy_desc(obs_dim, act_dim, 64, 2, cont)
+    _, named = random_policy(obs_dim, act_dim, hidden, layers, cont, seed=4)
+    desc = kernels.policy_desc(obs_dim, act_dim, hidden, layers, cont)
     flat = torch.from_numpy(flat_from_named(named)).cuda()
     B = 5000
     g = torch.Generator().manual_seed(2)

@@ -70,6 +70,71 @@ def test_update_step(golden_dir, tag):
                                    [-0.0097216293, 0.4503803849, 0.6908517480, 0.2085600495, 1.0845984221], rtol=2e-5)
 
 
+def _golden_update_case(golden_dir, file, tag):
+    """(named initial parameters, continuous, inputs, loss options, max_grad_norm, lr, {step: (grads, stats, params) of the
+    reference}) of one case of update.npz / update_wide.npz; grads and params are (flat values, mask of the flat entries they
+    hold or None for all), params None where the file keeps no parameters after that step."""
+    from tests.helpers import flat_from_named, golden_flat
+    g = np.load(os.path.join(golden_dir, file))
+    names = [str(n) for n in g[f"{tag}_names"]]
+    if file == "update.npz":
+        named0 = {n: g[f"{tag}_p0_{n}"] for n in names}
+        clip, ent_c, vf_c, mgn, lr, norm_adv, clip_vloss = [float(v) for v in g[f"{tag}_hyper"]]
+        params = {s: (flat_from_named({n: g[f"{tag}_s{s}_p_{n}"] for n in names}), None) for s in range(2)}
+    else:
+        named0 = {}
+        for i, n in enumerate(names):
+            shape = tuple(int(v) for v in g[f"{tag}_pshape_{n}"])
+            k = np.arange(int(np.prod(shape)), dtype=np.float64)
+            named0[n] = torch.from_numpy(0.1 * np.sin(0.37 * k + i)).to(torch.float32).numpy().reshape(shape)
+        clip, ent_c, vf_c, mgn, lr = [float(v) for v in g[f"{tag}_hyper"]]
+        norm_adv, clip_vloss = 1.0, 1.0
+        params = {1: golden_flat(g, tag, "final_p", names)}
+    hyper = dict(clip_coeff=clip, ent_c=ent_c, vf_c=vf_c, norm_adv=bool(norm_adv), clip_vloss=bool(clip_vloss))
+    want = {}
+    for s in range(2):
+        if file == "update.npz":
+            grads = (flat_from_named({n: g[f"{tag}_s{s}_g_{n}"] for n in names}), None)
+        else:
+            grads = golden_flat(g, tag, f"s{s}_g", names)
+        want[s] = (grads, g[f"{tag}_s{s}_stats"], params.get(s))
+    inputs = [_t(g[f"{tag}_{k}"]) for k in ("obs", "act", "oldlp", "adv", "ret", "vold")]
+    return named0, "actor_logstd" in names, inputs, hyper, mgn, lr, want
+
+
+@pytest.mark.parametrize("file,tag", [("update.npz", t) for t in ("disc", "disc_big", "cont", "disc_nonorm", "disc_novclip")] +
+                         [("update_wide.npz", t) for t in ("disc128", "cont128", "disc128x3")])
+def test_float64_restatement_agrees_with_the_reference(golden_dir, file, tag):
+    """RefPolicy(dtype=float64): the float64 update the wide-kernel tests measure against must sit within the project's bars
+    of the reference's own fp32 gradients, stats and parameters (so it is the same computation, only more precise)."""
+    from tests.helpers import flat_from_named
+    named0, cont, inputs, hyper, mgn, lr, want = _golden_update_case(golden_dir, file, tag)
+    pol = R.RefPolicy(named0, cont, dtype=torch.float64)
+    opt = R.RefAdam(pol.tensors(), lr=lr, eps=1e-5)
+    inputs = [x if i == 1 and not cont else x.double() for i, x in enumerate(inputs)]
+    order = ("policy_loss", "value_loss", "entropy", "loss", "old_approx_kl", "approx_kl", "clipfrac", "grad_norm")
+    for step in range(2):
+        stats, raw, _, _ = R.ppo_update_step(pol, opt, *inputs, max_grad_norm=mgn, **hyper)
+        (gw, gsel), st_want, p_want = want[step]
+        got = flat_from_named({n: r.numpy() for n, r in zip(pol.p.keys(), raw)}, np.float64)
+        got = got if gsel is None else got[gsel]
+        l2 = float(np.linalg.norm(got - gw) / np.linalg.norm(gw))
+        st = np.array([stats[k] for k in order])
+        st_rel = float(np.max(np.abs(st - st_want) / np.maximum(np.abs(st_want), 1e-30)))
+        msg = f"{file} {tag} step {step}: float64 vs the reference's fp32 gradients rel L2 {l2:.2e}, stats max rel {st_rel:.2e}"
+        if p_want is not None:
+            pw, psel = p_want
+            p64 = flat_from_named({n: t.detach().numpy() for n, t in pol.p.items()}, np.float64)
+            p64 = p64 if psel is None else p64[psel]
+            msg += f", parameters max abs {float(np.abs(p64 - pw).max()):.2e}"
+        print(msg)
+        np.testing.assert_allclose(got, gw, rtol=1e-4, atol=1e-4 * float(np.abs(gw).max()) + 1e-9)
+        assert l2 < 1e-4
+        np.testing.assert_allclose(st, st_want, rtol=1e-4, atol=2e-6)
+        if p_want is not None:
+            np.testing.assert_allclose(p64, pw, rtol=1e-5, atol=1e-6)
+
+
 def test_squashed_sample(golden_dir):
     g = np.load(os.path.join(golden_dir, "squash.npz"))
     x, act = _t(g["x"]), _t(g["act"])

@@ -128,11 +128,21 @@ def test_cartpole_replay_is_bit_exact(N, T):
     np.testing.assert_allclose(buf.next_value[sub].cpu().numpy(), nv.numpy(), **TOL)
 
 
-@pytest.mark.parametrize("N,T", [(7, 450), (300, 256)])
-def test_mountaincar_replay_is_bit_exact(N, T):
+# N, T, hidden, layers.  Past 64 x 2 each width is the first MountainCar-v0 run of its kernels: 128 x 2 takes
+# rollout_tc_kernel<MountainCar, 128> + critic_values_tc_kernel<128> with 2 observations; 256 x 2 and 128 x 3 take the
+# layer-wise actor (rollout_wide.cu) and rollout_tc_kernel<MountainCar, 0>, the external-actor mode with 3 logits; simt takes
+# the runtime-width kernel at 128 / 256 units
+MOUNTAINCAR_REPLAYS = {"7-450": (7, 450, 64, 2), "300-256": (300, 256, 64, 2), "128x2": (300, 256, 128, 2),
+                       "256x2": (130, 256, 256, 2), "128x3": (130, 256, 128, 3)}
+
+
+@pytest.mark.parametrize("case", list(MOUNTAINCAR_REPLAYS))
+def test_mountaincar_replay_is_bit_exact(case, rollout_impl):
     """MountainCar-v0 ((f) rank 4: more classic-control envs behind --gym_id): obs 2, 3 discrete actions, TimeLimit 200."""
-    pol, named = random_policy(2, 3, 64, 2, False, seed=8)
-    desc = kernels.policy_desc(2, 3, 64, 2, False)
+    N, T, hidden, layers = MOUNTAINCAR_REPLAYS[case]
+    L = _lib.lib()
+    pol, named = random_policy(2, 3, hidden, layers, False, seed=8)
+    desc = kernels.policy_desc(2, 3, hidden, layers, False)
     flat = torch.from_numpy(flat_from_named(named)).cuda()
     seeds = list(range(N))
     rng = np.random.default_rng(N)
@@ -143,8 +153,11 @@ def test_mountaincar_replay_is_bit_exact(N, T):
     o, _ = env.reset(seeds)
     assert np.array_equal(o.cpu().numpy(), obs0)
     buf = kernels.RolloutBuffers(T, N, 2, (), "cuda")
+    L.aur_launch_count_reset()
     kernels.rollout(env, desc, flat, buf, seed=1, step0=0, actions_in=torch.from_numpy(actions.astype(np.float32)).cuda())
     torch.cuda.synchronize()
+    layerwise = rollout_impl == "tc" and (hidden, layers) not in ((64, 2), (128, 2))
+    assert (L.aur_launch_count() >= T) == layerwise          # the layer-wise actor launches per step, a fused rollout does not
     assert np.array_equal(buf.states.cpu().numpy(), obs)
     assert np.array_equal(buf.terminals.cpu().numpy(), done)
     assert np.array_equal(buf.rewards.cpu().numpy(), rew)
@@ -157,8 +170,10 @@ def test_mountaincar_replay_is_bit_exact(N, T):
     ot = torch.from_numpy(obs[:, sub].reshape(-1, 2)); at = torch.from_numpy(actions[:, sub].reshape(-1))
     with torch.no_grad():
         _, lp, _, v = pol.evaluate(ot, at)
+        nv = pol.value(torch.from_numpy(last_obs[sub]))
     np.testing.assert_allclose(buf.log_probs[:, sub].cpu().numpy().reshape(-1), lp.numpy(), **TOL)
     np.testing.assert_allclose(buf.values[:, sub].cpu().numpy().reshape(-1), v.numpy().reshape(-1), **TOL)
+    np.testing.assert_allclose(buf.next_value[sub].cpu().numpy(), nv.numpy(), **TOL)
 
 
 def _oracle_replay_adaptive(kind, N, seeds, actions, T):

@@ -121,6 +121,8 @@ ROLLOUTS = {
     "cartpole-256x2": ("CartPole-v1", 4, 2, 256, 2, False, False, 2048, 8, True),     # tc: layer-wise actor (rollout_wide.cu)
     "cartpole-32x3": ("CartPole-v1", 4, 2, 32, 3, False, False, 2048, 12, False),
     "mountaincar": ("MountainCar-v0", 2, 3, 64, 2, False, False, 2048, 12, True),
+    "mountaincar-128x2": ("MountainCar-v0", 2, 3, 128, 2, False, False, 2048, 12, True),   # tc: rollout_tc_kernel<MountainCar, 128>
+    "mountaincar-256x2": ("MountainCar-v0", 2, 3, 256, 2, False, False, 2048, 8, True),    # tc: 3-class draws, external-actor mode
     "acrobot": ("Acrobot-v1", 6, 3, 64, 2, False, False, 2048, 12, False),
     "pendulum-wrappers": ("Pendulum-v1", 3, 1, 64, 2, True, True, 2048, 12, True),
     "pendulum": ("Pendulum-v1", 3, 1, 64, 2, True, False, 2048, 12, True),
@@ -140,7 +142,11 @@ def test_sampled_rollout_draws_follow_the_restatement(case, rollout_impl):
     env = denv.DeviceVecEnv(gym_id, N, wrappers=wrappers, env_id0=env_id0)
     env.reset(list(range(N)))
     buf = kernels.RolloutBuffers(T, N, obs_dim, (A,) if cont else (), "cuda")
+    L = _lib.lib()
+    L.aur_launch_count_reset()
     kernels.rollout(env, desc, flat, buf, seed=seed, step0=step0)
+    layerwise = rollout_impl == "tc" and hidden in (128, 256) and (hidden, layers) != (128, 2)
+    assert (L.aur_launch_count() >= T) == layerwise          # the layer-wise actor launches per step, a fused rollout does not
     head = _mlp64(named, "actor", buf.states.cpu().numpy().reshape(-1, obs_dim))
     gid = (np.uint64(env_id0) + np.arange(N, dtype=np.uint64))[None, :].repeat(T, 0).reshape(-1)
     step = (np.uint64(step0) + np.arange(T, dtype=np.uint64)).repeat(N)

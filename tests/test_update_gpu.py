@@ -108,28 +108,33 @@ def test_update_with_shuffled_gather_vs_oracle(cont, m, B):
                                    rtol=1e-5, atol=1e-6)
 
 
-def test_identity_index_range_and_split_minibatch():
+def test_identity_index_range_and_split_minibatch(update_impl):
     """idx=NULL + offset equals an explicit arange; two half-minibatch gradient buffers summed
-    equal the whole (the data-parallel contract: m_total scales, partial sums add)."""
-    pol, named = random_policy(4, 2, 64, 2, False, seed=12)
-    desc = kernels.policy_desc(4, 2, 64, 2, False)
-    g = torch.Generator().manual_seed(2)
-    B = 2048
-    bufs = [torch.randn(B, 4, generator=g), torch.randint(0, 2, (B,), generator=g).float(), -0.7 + 0.2 * torch.randn(B, generator=g),
-            torch.randn(B, generator=g), torch.randn(B, generator=g), torch.randn(B, generator=g)]
-    dbuf = [t.cuda() for t in bufs]
-    params = torch.from_numpy(flat_from_named(named)).cuda()
-    up = kernels.Updater(desc, params)
-    full = up.grad(*dbuf, torch.arange(512, 1536, dtype=torch.int32, device="cuda")).clone()
-    rng = up.grad(*dbuf, None, idx_offset=512, m_local=1024).clone()
-    assert torch.equal(full, rng)
-    # halves: moments must be the whole minibatch's, so feed them through the allreduce hook
-    whole_moments = up.moments.clone()
-    up.allreduce = lambda t: t.copy_(whole_moments) if t.dtype == torch.float64 else None
-    a = up.grad(*dbuf, None, idx_offset=512, m_local=512, m_total=1024).clone()
-    b = up.grad(*dbuf, None, idx_offset=1024, m_local=512, m_total=1024).clone()
-    np.testing.assert_allclose((a + b)[:up.P].cpu().numpy(), full[:up.P].cpu().numpy(), rtol=2e-5, atol=1e-8)
-    np.testing.assert_allclose((a + b)[up.P:up.P + 6].cpu().numpy(), full[up.P:up.P + 6].cpu().numpy(), rtol=1e-5)
+    equal the whole (the data-parallel contract: m_total scales, partial sums add).  Besides 64 x 2, the layer-wise wide
+    update (update_wide.cu) at 128 x 2 and at 256 x 3 (a middle layer): the first runs of its idx = NULL + idx_offset gather
+    and of an m_total other than m_local there; they do not depend on update_impl, so they run once."""
+    shapes = [(4, 2, 64, 2)] + ([(4, 2, 128, 2), (6, 3, 256, 3)] if update_impl == "tc" else [])
+    for obs_dim, act_dim, hidden, layers in shapes:
+        _, named = random_policy(obs_dim, act_dim, hidden, layers, False, seed=12)
+        desc = kernels.policy_desc(obs_dim, act_dim, hidden, layers, False)
+        g = torch.Generator().manual_seed(2)
+        B = 2048
+        bufs = [torch.randn(B, obs_dim, generator=g), torch.randint(0, act_dim, (B,), generator=g).float(),
+                -0.7 + 0.2 * torch.randn(B, generator=g), torch.randn(B, generator=g), torch.randn(B, generator=g),
+                torch.randn(B, generator=g)]
+        dbuf = [t.cuda() for t in bufs]
+        params = torch.from_numpy(flat_from_named(named)).cuda()
+        up = kernels.Updater(desc, params)
+        full = up.grad(*dbuf, torch.arange(512, 1536, dtype=torch.int32, device="cuda")).clone()
+        rng = up.grad(*dbuf, None, idx_offset=512, m_local=1024).clone()
+        assert torch.equal(full, rng), hidden
+        # halves: moments must be the whole minibatch's, so feed them through the allreduce hook
+        whole_moments = up.moments.clone()
+        up.allreduce = lambda t: t.copy_(whole_moments) if t.dtype == torch.float64 else None
+        a = up.grad(*dbuf, None, idx_offset=512, m_local=512, m_total=1024).clone()
+        b = up.grad(*dbuf, None, idx_offset=1024, m_local=512, m_total=1024).clone()
+        np.testing.assert_allclose((a + b)[:up.P].cpu().numpy(), full[:up.P].cpu().numpy(), rtol=2e-5, atol=1e-8, err_msg=str(hidden))
+        np.testing.assert_allclose((a + b)[up.P:up.P + 6].cpu().numpy(), full[up.P:up.P + 6].cpu().numpy(), rtol=1e-5, err_msg=str(hidden))
 
 
 def test_large_minibatch_properties():
