@@ -369,10 +369,8 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
     tc::fence_after_sync();
     float2 h2[FP2];
 #pragma unroll
-    for (int c = 0; c < CPT; ++c) {
-      tc::tmem_ld8_nowait(tm_z + lane_base + (uint32_t)(f0 + 8 * c), h2 + 4 * c);
-      tc::tmem_wait_ld();
-    }
+    for (int c = 0; c < CPT; ++c) tc::tmem_ld8_nowait(tm_z + lane_base + (uint32_t)(f0 + 8 * c), h2 + 4 * c);
+    tc::tmem_wait_ld();                                // one round trip for all CPT chunks (their registers are h2 anyway)
     const float2 prescale2 = make_float2(TANH_PRESCALE, TANH_PRESCALE);
 #pragma unroll
     for (int g = 0; g < FPT / 4; ++g) {
@@ -501,10 +499,8 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
     __syncthreads();
     if (TPS == 4) {
 #pragma unroll
-      for (int c = 0; c < CPT; ++c) {
-        tc::tmem_ld8_nowait(tm_z + lane_base + (uint32_t)(f0 + 8 * c), h2 + 4 * c);
-        tc::tmem_wait_ld();
-      }
+      for (int c = 0; c < CPT; ++c) tc::tmem_ld8_nowait(tm_z + lane_base + (uint32_t)(f0 + 8 * c), h2 + 4 * c);
+      tc::tmem_wait_ld();
     }
     float dout[POL_OUT_MAX];
 #pragma unroll
@@ -557,6 +553,11 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
 #pragma unroll
         for (int j = 0; j < 4; ++j) { patch[2 * j * 36 + lane] = h2[4 * p + j].x; patch[(2 * j + 1) * 36 + lane] = h2[4 * p + j].y; }
       };
+      // this octet's dout, loaded once for all passes (TPS 2; TPS 4 has no registers to spare and reloads it per pass)
+      constexpr int KD = TPS == 2 ? OUT : 1;
+      float4 dva[KD], dvb[KD];
+#pragma unroll
+      for (int k = 0; k < KD; ++k) { dva[k] = lds4(dbase + k * T2_LD); dvb[k] = lds4(dbase + k * T2_LD + 4); }
       put(0);
       __syncwarp();
 #pragma unroll
@@ -567,7 +568,7 @@ __device__ __forceinline__ void tc_update_net(const UpdDev& a, const PopUpd& pop
 #pragma unroll
         for (int k = 0; k < POL_OUT_MAX; ++k) {
           if (k < OUT) {
-            const float4 da = lds4(dbase + k * T2_LD), db = lds4(dbase + k * T2_LD + 4);
+            const float4 da = TPS == 2 ? dva[k < KD ? k : 0] : lds4(dbase + k * T2_LD), db = TPS == 2 ? dvb[k < KD ? k : 0] : lds4(dbase + k * T2_LD + 4);
             float2 s01 = __fmul2_rn(make_float2(ha.x, ha.y), make_float2(da.x, da.y));      // even / odd samples
             s01 = __ffma2_rn(make_float2(ha.z, ha.w), make_float2(da.z, da.w), s01);
             s01 = __ffma2_rn(make_float2(hb.x, hb.y), make_float2(db.x, db.y), s01);
